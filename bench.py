@@ -1,6 +1,7 @@
 """bench.py -- the driver's measurement contract for the PLNLP hot path on B200.
 
   python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload citation2|ddi|collab]
+                  [--dump-outputs DIR]
 
 A "step" is one optimisation step of ``BaseModel.train`` over one batch of 65 536 positive edges and
 their negatives: full-graph encode (fwd + bwd), fused edge scoring + pairwise loss, clip, Adam.
@@ -20,6 +21,9 @@ the N = 1 line.
   roofline / kernels : per-kernel CUDA-event durations from an instrumented pass of the same K steps.
   cpu_baseline : the oracle restatement of the reference step (torch CPU, all host threads) on a
           bounded sample of the same workload.
+
+--dump-outputs DIR writes, after the timed steps, what the last of them left for its caller (``dump_outputs``) as
+DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -34,6 +38,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 
 import torch  # noqa: E402
 
@@ -138,6 +143,41 @@ def make_model(cfg, device):
                   optimizer_name="Adam", device=device, use_node_feats=cfg["use_feats"], train_node_emb=True)
     m.param_init()
     return m
+
+
+DUMP_TENSOR_BYTES = 8 << 20      # a larger [rows, cols] tensor is dumped as a fixed sample of its rows
+DUMP_TOTAL_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, model, loss_sum):
+    """--dump-outputs: what the last timed step left for the caller of the batch loop, as <out_dir>/<name>.npy --
+    ``loss_sum`` (float64: the batch loop's return value, sum of loss x batch size over the timed steps) and, in
+    float32, every parameter after that step's Adam update (``param.<name>``) and the gradient the update used
+    (``grad.<name>``; post-clip for the encoder and predictor).  A tensor over DUMP_TENSOR_BYTES (the node
+    embedding) keeps the rows ``sorted(torch.randperm(rows, generator seeded 0)[:n])``, the same rows for the
+    parameter and its gradient.  Multi-GPU: rank 0's tensors (its row block of the embedding)."""
+    import numpy as np
+    tensors = {"loss_sum": loss_sum.detach().double().reshape(1)}
+    named = [(prefix + n, p) for prefix, mod in (("emb.", model.emb), ("encoder.", model.encoder),
+                                                 ("predictor.", model.predictor)) if mod is not None
+             for n, p in mod.named_parameters()]
+    for name, p in named:
+        for kind, t in (("param", p), ("grad", p.grad)):
+            if t is None:
+                continue
+            t = t.detach().float()
+            if t.dim() == 2 and t.numel() * 4 > DUMP_TENSOR_BYTES:
+                n = DUMP_TENSOR_BYTES // (4 * t.size(1))
+                rows = torch.randperm(t.size(0), generator=torch.Generator().manual_seed(0))[:n].sort().values
+                t = t[rows.to(t.device)]
+            tensors[f"{kind}.{name}"] = t
+    arrays = {name: t.cpu().numpy() for name, t in tensors.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_TOTAL_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_TOTAL_BYTES}-byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -280,8 +320,8 @@ def measure(args, workload, world, rank, device, full):
                                      neg_sampler_name=cfg["sampler"], num_neg=k, device=device)
         model.encoder.train(); model.predictor.train()
         # the batch loop of BaseModel.train (index work of batch i + 1 prepared on a side stream while batch i runs)
-        model.run_batches(data, ((pos[i * Bl:(i + 1) * Bl], neg[i * Bl:(i + 1) * Bl].reshape(-1, 2),
-                                  None if wgt is None else wgt[i * Bl:(i + 1) * Bl]) for i in range(n)), k)
+        return model.run_batches(data, ((pos[i * Bl:(i + 1) * Bl], neg[i * Bl:(i + 1) * Bl].reshape(-1, 2),
+                                         None if wgt is None else wgt[i * Bl:(i + 1) * Bl]) for i in range(n)), k)
 
     out = {"cfg": cfg, "E": E, "partitioned": partitioned, "strong": strong, "K": K, "W": W}
 
@@ -320,7 +360,7 @@ def measure(args, workload, world, rank, device, full):
     clk.mark(True)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    device_steps(K, 1)
+    timed = device_steps(K, 1)
     e1.record()
     barrier()
     gc.enable()
@@ -328,6 +368,8 @@ def measure(args, workload, world, rank, device, full):
     clk.stop()
     ms = max_over_ranks(e0.elapsed_time(e1))
     out["launches"] = _lib.launch_count() - l0
+    if full and rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, model, timed[0])
     # host side of the same K steps: how long python + the launch calls take to ENQUEUE them (no device wait).  When
     # this approaches ms_per_step the run is launch-bound, not kernel-bound
     torch.cuda.synchronize()
@@ -572,7 +614,7 @@ def cpu_baseline_guarded(workload, steps, timeout_s=None):
     last = "no attempt"
     for threads in (0, 8):
         try:
-            r = subprocess.run([sys.executable, "-c", code, workload, str(steps), str(threads)], cwd=ROOT,
+            r = subprocess.run([sys.executable, "-B", "-c", code, workload, str(steps), str(threads)], cwd=ROOT,
                                capture_output=True, text=True, timeout=timeout_s)
             for ln in r.stdout.splitlines():
                 if ln.startswith("CPU_BASELINE "):
@@ -673,7 +715,13 @@ def main():
                     help="steps of the CPU arm's bounded sample (default: ~10-20 s of CPU work: one 17-batch epoch of "
                          "the ddi / collab shape, 2 steps of the citation2 shape)")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.cpu_steps is None:
         args.cpu_steps = 2 if args.workload == "citation2" else 17
     # the contract is ONE JSON line on stdout: keep a private handle to the real stdout and point fd 1

@@ -1,6 +1,5 @@
 """GPU test (-m gpu): the call sequence of the reference's main.py (main.py:70-266) through plnlp_b200.shims on tiny
-synthetic OGB-shape datasets -- dataset, ToSparseTensor, graph preparation, data.to(device), BaseModel, train, test.
-(The real main.py is executed through the same shims by tests/test_shims_cpu.py, up to the model, on the CPU box.)"""
+synthetic OGB-shape datasets -- dataset, ToSparseTensor, graph preparation, data.to(device), BaseModel, train, test."""
 import pytest
 import torch
 
