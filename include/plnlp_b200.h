@@ -338,6 +338,30 @@ int plnlp_mrr_counts_f32(const float* pos, const float* neg, int64_t ldn, int64_
                          int32_t* gt, int32_t* ge, void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * Link recommendation over all nodes (csrc/topk.cu; an extension, no reference call site): a score chunk
+ * s [Q, N] holds row q = the predictor scores of (node[q], j) for every candidate j.
+ */
+/* Known-link filter: s[q*lds + col[e]] = -inf for e in [rowptr[node[q]], rowptr[node[q]+1]);
+ * when exclude_self != 0, also s[q*lds + node[q]] = -inf.  Columns outside [0, N) are ignored.
+ * rowptr == col == NULL: no known links (self only).  node[q] must be a row of the CSR (the caller's promise). */
+int plnlp_score_mask_f32(float* s, int64_t lds, int64_t Q, int64_t N, const int64_t* node,
+                         const int64_t* rowptr, const int32_t* col, int exclude_self, void* stream);
+
+/* Per row q of s [Q, N] (row-major, lds >= N):
+ *  - 0 < k <= 1024: the k largest finite entries, by score descending then column ascending
+ *    -> ids [Q, k], scores [Q, k]; the tail is (-1, -inf) when fewer than k are finite.  -0 ties with +0.
+ *  - target != NULL: gt[q] / ge[q] = #{j != target[q], s_j finite, s_j > / >= target_score[q]}.
+ *    target_score is read by the caller BEFORE masking.
+ * k == 0 with ids == NULL: rank counts only.  k > 1024 is PLNLP_E_UNSUPPORTED, N >= 2^31 PLNLP_E_SIZE.
+ * One read of s.  Deterministic; integer outputs are exact.
+ * workspace: plnlp_topk_rows_workspace_bytes(Q, N, k) bytes, 16-byte aligned. */
+int64_t plnlp_topk_rows_workspace_bytes(int64_t Q, int64_t N, int64_t k);
+int plnlp_topk_rows_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t k,
+                        const int64_t* target, const float* target_score,
+                        int64_t* ids, float* scores, int32_t* gt, int32_t* ge,
+                        void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Random-walk augmentation (SURVEY.md 8f rank 1; replaces torch_cluster.random_walk and the pair /
  * weight assembly of main.py:228-233, 241-253).  rowptr / col: the reference's int64 CSR arrays.
  */

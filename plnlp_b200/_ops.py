@@ -1137,3 +1137,49 @@ def mrr_counts_raw(pos, neg):
     check(lib.plnlp_mrr_counts_f32(ptr(pos), ptr(neg), _ld(neg), S, K, ptr(gt), ptr(ge), stream()),
           "plnlp_mrr_counts_f32")
     return gt, ge
+
+
+def score_mask_raw(s, nodes, rowptr=None, col=None, exclude_self=True):
+    """in place: s[q, j] = -inf for the known links j of nodes[q] (CSR rowptr int64 / col int32) and, with
+    ``exclude_self``, for j = nodes[q]"""
+    lib = _lib.load()
+    if _f32c(s).dim() != 2 or s.stride(1) != 1:
+        raise RuntimeError("the score chunk must be a 2-D fp32 matrix with unit column stride (masked in place)")
+    nodes = nodes.contiguous()
+    if nodes.dtype != torch.int64 or nodes.numel() != s.size(0):
+        raise RuntimeError("nodes must be int64 with one entry per score row")
+    if (rowptr is None) != (col is None):
+        raise RuntimeError("rowptr and col come together")
+    if col is not None and (rowptr.dtype != torch.int64 or col.dtype != torch.int32):
+        raise RuntimeError("the known-link CSR is int64 rowptr + int32 col")
+    Q, N = s.shape
+    with profiling.span("score_mask_f32", 0, 0):
+        check(lib.plnlp_score_mask_f32(ptr(s), _ld(s), Q, N, ptr(nodes), ptr(rowptr), ptr(col), int(bool(exclude_self)),
+                                       stream()), "plnlp_score_mask_f32")
+    return s
+
+
+def topk_rows_raw(s, k, target=None, target_score=None):
+    """per row of s [Q, N]: the k largest finite entries (score descending, then column ascending; tail (-1, -inf))
+    and, with ``target``, the filtered rank counts gt / ge against ``target_score``.  -> (ids int64 [Q, k] or None,
+    scores [Q, k] or None, gt int32 [Q] or None, ge int32 [Q] or None).  One read of s."""
+    lib = _lib.load()
+    s = _rowmajor(s)
+    Q, N = s.shape
+    dev = s.device
+    ids = torch.empty(Q, k, dtype=torch.int64, device=dev) if k > 0 else None
+    scores = torch.empty(Q, k, dtype=torch.float32, device=dev) if k > 0 else None
+    gt = ge = None
+    if target is not None:
+        target = target.contiguous()
+        target_score = _f32c(target_score).contiguous()
+        if target.dtype != torch.int64 or target.numel() != Q or target_score.numel() != Q:
+            raise RuntimeError("target (int64) and target_score need one entry per score row")
+        gt = torch.empty(Q, dtype=torch.int32, device=dev)
+        ge = torch.empty(Q, dtype=torch.int32, device=dev)
+    nbytes = max(int(lib.plnlp_topk_rows_workspace_bytes(Q, N, max(int(k), 0))), 16)
+    ws = workspace.get("topk_rows", nbytes, dev)
+    with profiling.span(f"topk_rows_f32 k={k}", Q * N * 4, 0):
+        check(lib.plnlp_topk_rows_f32(ptr(s), _ld(s), Q, N, int(k), ptr(target), ptr(target_score), ptr(ids),
+                                      ptr(scores), ptr(gt), ptr(ge), ptr(ws), nbytes, stream()), "plnlp_topk_rows_f32")
+    return ids, scores, gt, ge

@@ -92,6 +92,16 @@ def evaluate_mrr(evaluator, pos_val_pred, neg_val_pred, pos_test_pred, neg_test_
     return {'MRR': (mrr_list(pv, nv).mean().item(), mrr_list(pt, nt).mean().item())}
 
 
+def full_rank_metrics(ranks, ks=(1, 3, 10, 20, 50, 100)):
+    """MRR and Hits@K of full-ranking ranks (``BaseModel.rank_against_all``): mean of 1 / rank and the fraction of
+    ranks <= K, computed on the GPU with one host read -> {'MRR': float, 'Hits@K': float, ...}"""
+    r = _cuda_f32(ranks).reshape(-1)
+    vals = torch.stack([r.reciprocal().mean()] + [(r <= K).to(torch.float32).mean() for K in ks]).tolist()
+    out = {'MRR': vals[0]}
+    out.update({f'Hits@{K}': v for K, v in zip(ks, vals[1:])})
+    return out
+
+
 def gcn_normalization(adj_t):
     """utils.py:83-89: D^-1/2 (A + I) D^-1/2 with inf -> 0, on whatever adjacency type is given
     (CSRGraph or torch_sparse.SparseTensor: only set_diag / sum / broadcast-mul are used)."""
