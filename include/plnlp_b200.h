@@ -361,6 +361,23 @@ int plnlp_topk_rows_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64
                         int64_t* ids, float* scores, int32_t* gt, int32_t* ge,
                         void* workspace, int64_t workspace_bytes, void* stream);
 
+/* Column-offset forms for one shard of the candidates: s [Q, N] covers the global candidate ids [col0, col0 + N)
+ * (0 <= col0, col0 + N < 2^31, else PLNLP_E_SIZE).  The mask reads col[] and node[q] as global ids (a known link c
+ * lands at column c - col0); the select reports global ids col0 + j, breaks ties on them and compares target[q]
+ * with them.  plnlp_score_mask_f32 / plnlp_topk_rows_f32 are these with col0 = 0. */
+int plnlp_score_mask_cols_f32(float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, const int64_t* node,
+                              const int64_t* rowptr, const int32_t* col, int exclude_self, void* stream);
+int plnlp_topk_rows_cols_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, int64_t k,
+                             const int64_t* target, const float* target_score,
+                             int64_t* ids, float* scores, int32_t* gt, int32_t* ge,
+                             void* workspace, int64_t workspace_bytes, void* stream);
+/* Cross-shard merge: ids_in / scores_in [R, Q, k_in] (rank-major: the all-gather of R per-shard [Q, k_in] results)
+ * -> ids / scores [Q, k] (1 <= k <= 1024): per row the k best entries of the R lists by score descending then id
+ * ascending, the tail (-1, -inf).  An entry with id < 0 or a non-finite score is dead.  Keys are rebuilt from
+ * (score, global id), so the result does not depend on R or on how the candidates were split. */
+int plnlp_topk_merge_f32(const int64_t* ids_in, const float* scores_in, int64_t R, int64_t Q, int64_t k_in,
+                         int64_t k, int64_t* ids, float* scores, void* stream);
+
 /* ------------------------------------------------------------------------------------
  * Random-walk augmentation (SURVEY.md 8f rank 1; replaces torch_cluster.random_walk and the pair /
  * weight assembly of main.py:228-233, 241-253).  rowptr / col: the reference's int64 CSR arrays.

@@ -62,6 +62,9 @@ SIGNATURES = {
     "plnlp_score_mask_f32": (c_int, [_P, _L, _L, _L, _P, _P, _P, _I, _P]),
     "plnlp_topk_rows_workspace_bytes": (c_int64, [_L, _L, _L]),
     "plnlp_topk_rows_f32": (c_int, [_P, _L, _L, _L, _L, _P, _P, _P, _P, _P, _P, _P, _L, _P]),
+    "plnlp_score_mask_cols_f32": (c_int, [_P, _L, _L, _L, _L, _P, _P, _P, _I, _P]),
+    "plnlp_topk_rows_cols_f32": (c_int, [_P, _L, _L, _L, _L, _L, _P, _P, _P, _P, _P, _P, _P, _L, _P]),
+    "plnlp_topk_merge_f32": (c_int, [_P, _P, _L, _L, _L, _L, _P, _P, _P]),
     "plnlp_graph_make_keys": (c_int, [_P, _P, _L, _L, _I, _I, _P, _P, _P]),
     "plnlp_graph_diag_keys": (c_int, [_L, _L, _P, _P, _L, _P]),
     "plnlp_graph_sort_workspace_bytes": (c_int64, [_L]),

@@ -155,8 +155,10 @@ def spmm_raw(plan, x, use_val, div_rows, bias=None, relu=False, drop_p=0.0, seed
 
 
 def gemm_raw(A, B, transa=False, transb=False, C=None, beta=0.0, bias=None, act=ACT_NONE, aux=None,
-             drop_p=0.0, seed=0, split_k=None, backend=None):
-    """C = act(op(A) @ op(B) + beta*C + bias); A, B row-major with leading dimensions."""
+             drop_p=0.0, seed=0, split_k=None, backend=None, fixed_backend=False):
+    """C = act(op(A) @ op(B) + beta*C + bias); A, B row-major with leading dimensions.  ``fixed_backend``: run
+    ``backend`` itself, whatever the shape (no switch to the CUDA-core kernel for a small product, no TMA-fed
+    kernel): for a caller whose results must not depend on the row count of A."""
     lib = _lib.load()
     A, B = _rowmajor(A), _rowmajor(B)
     M, K = (A.size(1), A.size(0)) if transa else (A.size(0), A.size(1))
@@ -167,7 +169,7 @@ def gemm_raw(A, B, transa=False, transb=False, C=None, beta=0.0, bias=None, act=
         C = torch.empty(M, N, dtype=torch.float32, device=A.device)
         beta = 0.0
     backend = backend or GEMM_BACKEND
-    if backend != "ffma" and (K < 32 or N < 16 or M * N * K < (1 << 20)):
+    if backend != "ffma" and not fixed_backend and (K < 32 or N < 16 or M * N * K < (1 << 20)):
         backend = "ffma"                      # too little work for a tensor-core tile (a small M x N with a
                                               # huge K -- weight gradients -- does go to the tensor cores)
     bn = 128 if backend == "ffma" or (N <= 128 and not backend.endswith("c2")) else 256
@@ -185,7 +187,8 @@ def gemm_raw(A, B, transa=False, transb=False, C=None, beta=0.0, bias=None, act=
     if split_k > 1:
         ws_bytes = split_k * M * N * 4
         ws = workspace.get("gemm_splitk", ws_bytes, A.device)
-    if (backend in ("tf32x3c2", "tf32c2", "tf32x3", "tf32") and GEMM_TMA != "0" and not transa and split_k == 1
+    if (backend in ("tf32x3c2", "tf32c2", "tf32x3", "tf32") and GEMM_TMA != "0" and not fixed_backend and not transa
+            and split_k == 1
             and K >= 32 and N <= 512 and _ld(A) % 4 == 0 and A.data_ptr() % 16 == 0
             and (GEMM_TMA == "1" or (M >= 16384 and N <= 256 and K <= 512))):
         nbytes = lib.plnlp_gemm_tf32_tma_workspace_bytes(N, K)
@@ -1139,9 +1142,10 @@ def mrr_counts_raw(pos, neg):
     return gt, ge
 
 
-def score_mask_raw(s, nodes, rowptr=None, col=None, exclude_self=True):
+def score_mask_raw(s, nodes, rowptr=None, col=None, exclude_self=True, col0=0):
     """in place: s[q, j] = -inf for the known links j of nodes[q] (CSR rowptr int64 / col int32) and, with
-    ``exclude_self``, for j = nodes[q]"""
+    ``exclude_self``, for j = nodes[q].  The chunk covers the global candidate ids [col0, col0 + N): col and nodes
+    are global ids."""
     lib = _lib.load()
     if _f32c(s).dim() != 2 or s.stride(1) != 1:
         raise RuntimeError("the score chunk must be a 2-D fp32 matrix with unit column stride (masked in place)")
@@ -1154,15 +1158,16 @@ def score_mask_raw(s, nodes, rowptr=None, col=None, exclude_self=True):
         raise RuntimeError("the known-link CSR is int64 rowptr + int32 col")
     Q, N = s.shape
     with profiling.span("score_mask_f32", 0, 0):
-        check(lib.plnlp_score_mask_f32(ptr(s), _ld(s), Q, N, ptr(nodes), ptr(rowptr), ptr(col), int(bool(exclude_self)),
-                                       stream()), "plnlp_score_mask_f32")
+        check(lib.plnlp_score_mask_cols_f32(ptr(s), _ld(s), Q, N, int(col0), ptr(nodes), ptr(rowptr), ptr(col),
+                                            int(bool(exclude_self)), stream()), "plnlp_score_mask_cols_f32")
     return s
 
 
-def topk_rows_raw(s, k, target=None, target_score=None):
+def topk_rows_raw(s, k, target=None, target_score=None, col0=0):
     """per row of s [Q, N]: the k largest finite entries (score descending, then column ascending; tail (-1, -inf))
     and, with ``target``, the filtered rank counts gt / ge against ``target_score``.  -> (ids int64 [Q, k] or None,
-    scores [Q, k] or None, gt int32 [Q] or None, ge int32 [Q] or None).  One read of s."""
+    scores [Q, k] or None, gt int32 [Q] or None, ge int32 [Q] or None).  One read of s.  The chunk covers the
+    global candidate ids [col0, col0 + N): ids, ties and ``target`` are global ids."""
     lib = _lib.load()
     s = _rowmajor(s)
     Q, N = s.shape
@@ -1180,6 +1185,23 @@ def topk_rows_raw(s, k, target=None, target_score=None):
     nbytes = max(int(lib.plnlp_topk_rows_workspace_bytes(Q, N, max(int(k), 0))), 16)
     ws = workspace.get("topk_rows", nbytes, dev)
     with profiling.span(f"topk_rows_f32 k={k}", Q * N * 4, 0):
-        check(lib.plnlp_topk_rows_f32(ptr(s), _ld(s), Q, N, int(k), ptr(target), ptr(target_score), ptr(ids),
-                                      ptr(scores), ptr(gt), ptr(ge), ptr(ws), nbytes, stream()), "plnlp_topk_rows_f32")
+        check(lib.plnlp_topk_rows_cols_f32(ptr(s), _ld(s), Q, N, int(col0), int(k), ptr(target), ptr(target_score),
+                                           ptr(ids), ptr(scores), ptr(gt), ptr(ge), ptr(ws), nbytes, stream()),
+              "plnlp_topk_rows_cols_f32")
     return ids, scores, gt, ge
+
+
+def topk_merge_raw(ids_in, scores_in, k):
+    """the k best entries per row of R sorted per-shard lists ids_in int64 / scores_in fp32 [R, Q, k_in] (dead
+    entries: id -1) -> (ids int64 [Q, k], scores [Q, k]) under the tie rule of ``topk_rows_raw``"""
+    lib = _lib.load()
+    if ids_in.dim() != 3 or ids_in.shape != scores_in.shape or ids_in.dtype != torch.int64:
+        raise RuntimeError("ids_in (int64) and scores_in must both be [R, Q, k_in]")
+    ids_in, scores_in = ids_in.contiguous(), _f32c(scores_in).contiguous()
+    R, Q, k_in = ids_in.shape
+    ids = torch.empty(Q, k, dtype=torch.int64, device=ids_in.device)
+    scores = torch.empty(Q, k, dtype=torch.float32, device=ids_in.device)
+    with profiling.span(f"topk_merge_f32 R={R}", ids_in.numel() * 12, 0):
+        check(lib.plnlp_topk_merge_f32(ptr(ids_in), ptr(scores_in), R, Q, k_in, int(k), ptr(ids), ptr(scores),
+                                       stream()), "plnlp_topk_merge_f32")
+    return ids, scores

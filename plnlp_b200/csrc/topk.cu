@@ -6,6 +6,10 @@
 // scores the lower column.  Every key of a row is distinct, so "the k largest keys" is exactly the top-k under
 // the tie rule (score descending, then column ascending) and every selection below is order independent.
 //
+// A chunk may cover the candidate columns [col0, col0 + N) of a wider id space (one shard of a row-partitioned
+// graph): keys, ids and the target comparison then use the global column col0 + j, so per-shard results merge
+// into exactly the selection over the whole row (topk_cross_merge_kernel).
+//
 // Two kernels, ONE pass over the score chunk:
 //   topk_segment_kernel  one CTA per (row, segment of kSeg columns).  Streams its segment once, counts gt / ge
 //                        against the target score, and keeps a candidate buffer in shared memory: an entry is
@@ -15,6 +19,8 @@
 //   topk_merge_kernel    one CTA per row: sums the counts, selects the k best of the segments' candidates (at most
 //                        ceil(N / kSeg) * k keys, L2 resident), sorts them (bitonic, shared memory) and writes ids
 //                        and scores.
+// plus topk_cross_merge_kernel: one CTA per row, the k best of R per-shard sorted lists (ids, scores), with the
+// select / sort / write tail of topk_merge_kernel.
 // Integer outputs are exact; ids / scores do not depend on the launch configuration.
 #include <cfloat>
 
@@ -143,17 +149,19 @@ __device__ void cut_to_k(SegShared& sh, int k) {
     __syncthreads();
 }
 
-// grid.x = Q * n_seg; CTA b handles row b / n_seg, columns [seg * kSeg, min(N, (seg + 1) * kSeg))
+// grid.x = Q * n_seg; CTA b handles row b / n_seg, global columns [col0 + seg * kSeg, min(col_end, ... + kSeg)).
+// s_shifted = s - col0 (formed as an address by the host), so the loop runs on global columns: the column offset
+// costs no register (the kernel stays at 62 registers, 4 CTAs per SM).
 __global__ void __launch_bounds__(kThreads, 4) topk_segment_kernel(
-    const float* __restrict__ s, int64_t lds, int64_t N, int k, int n_seg, const int64_t* __restrict__ target,
-    const float* __restrict__ target_score, uint64_t* __restrict__ cand, int* __restrict__ cand_n,
-    int* __restrict__ part_gt, int* __restrict__ part_ge) {
+    const float* __restrict__ s_shifted, int64_t lds, int64_t col0, int64_t col_end, int k, int n_seg,
+    const int64_t* __restrict__ target, const float* __restrict__ target_score, uint64_t* __restrict__ cand,
+    int* __restrict__ cand_n, int* __restrict__ part_gt, int* __restrict__ part_ge) {
     __shared__ SegShared sh;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t b = blockIdx.x;
     const int64_t q = b / n_seg;
-    const int64_t c0 = (b % n_seg) * kSeg, c1 = min(N, c0 + kSeg);
-    const float* row = s + q * lds;
+    const int64_t c0 = col0 + (b % n_seg) * kSeg, c1 = min(col_end, c0 + kSeg);
+    const float* row = s_shifted + q * lds;
     const bool rank = target != nullptr;
     const int64_t tcol = rank ? target[q] : -1;
     const float tval = rank ? target_score[q] : 0.0f;
@@ -224,36 +232,15 @@ struct MergeShared {
     int cnt;
 };
 
-// one CTA per row: gt / ge sums, then the k best of the n_seg * k candidate slots (slot i of segment g is live when
-// i < cand_n[g]; dead slots read as key 0, below every live key), sorted, written as (id, score)
-__global__ void __launch_bounds__(kThreads) topk_merge_kernel(
-    const uint64_t* __restrict__ cand, const int* __restrict__ cand_n, const int* __restrict__ part_gt,
-    const int* __restrict__ part_ge, int n_seg, int k, int64_t* __restrict__ ids, float* __restrict__ scores,
-    int32_t* __restrict__ gt, int32_t* __restrict__ ge) {
-    __shared__ MergeShared sh;
+// the tail of both merges, run by one CTA for one row: the k best of the keys get(0 .. slots) -- ``total`` of them
+// live, dead slots read as key 0, below every live key -- sorted descending (bitonic, shared memory) and written as
+// (id, score), the tail (-1, -inf).  Begins in sync.
+template <class Get>
+__device__ void select_sort_write(Get get, int slots, int total, int k, int64_t* __restrict__ ids,
+                                  float* __restrict__ scores, MergeShared& sh) {
     const int tid = threadIdx.x;
-    const int64_t q = blockIdx.x;
-    const int64_t g0 = q * n_seg;
-    if (gt != nullptr && tid == 0) {
-        int a = 0, c = 0;
-        for (int g = 0; g < n_seg; ++g) { a += part_gt[g0 + g]; c += part_ge[g0 + g]; }
-        gt[q] = a;
-        ge[q] = c;
-    }
-    if (k == 0) return;
-    if (tid == 0) {
-        int t = 0;
-        for (int g = 0; g < n_seg; ++g) t += cand_n[g0 + g];
-        sh.total = t;
-        sh.cnt = 0;
-    }
-    __syncthreads();
-    const uint64_t* rc = cand + g0 * k;
-    const int* rn = cand_n + g0;
-    const int slots = n_seg * k;
-    auto get = [rc, rn, k](int i) -> uint64_t { return (i % k) < __ldg(rn + i / k) ? __ldg(rc + i) : 0ull; };
-    const int m = min(sh.total, k);
-    const uint64_t kth = sh.total > k ? block_select(get, slots, k, sh.sel) : 1ull;
+    const int m = min(total, k);
+    const uint64_t kth = total > k ? block_select(get, slots, k, sh.sel) : 1ull;
     for (int i = tid; i < slots; i += kThreads) {
         const uint64_t key = get(i);
         if (key >= kth && key != 0ull) sh.buf[atomicAdd(&sh.cnt, 1)] = key;
@@ -278,16 +265,72 @@ __global__ void __launch_bounds__(kThreads) topk_merge_kernel(
     for (int i = tid; i < k; i += kThreads) {
         if (i < m) {
             const uint64_t key = sh.buf[i];
-            ids[q * k + i] = static_cast<int64_t>(~static_cast<uint32_t>(key));
-            scores[q * k + i] = key_float(static_cast<uint32_t>(key >> 32));
+            ids[i] = static_cast<int64_t>(~static_cast<uint32_t>(key));
+            scores[i] = key_float(static_cast<uint32_t>(key >> 32));
         } else {
-            ids[q * k + i] = -1;
-            scores[q * k + i] = -INFINITY;
+            ids[i] = -1;
+            scores[i] = -INFINITY;
         }
     }
 }
 
-__global__ void __launch_bounds__(128) score_mask_kernel(float* __restrict__ s, int64_t lds, int64_t N,
+// one CTA per row: gt / ge sums, then the k best of the n_seg * k candidate slots (slot i of segment g is live when
+// i < cand_n[g]), sorted, written as (id, score)
+__global__ void __launch_bounds__(kThreads) topk_merge_kernel(
+    const uint64_t* __restrict__ cand, const int* __restrict__ cand_n, const int* __restrict__ part_gt,
+    const int* __restrict__ part_ge, int n_seg, int k, int64_t* __restrict__ ids, float* __restrict__ scores,
+    int32_t* __restrict__ gt, int32_t* __restrict__ ge) {
+    __shared__ MergeShared sh;
+    const int tid = threadIdx.x;
+    const int64_t q = blockIdx.x;
+    const int64_t g0 = q * n_seg;
+    if (gt != nullptr && tid == 0) {
+        int a = 0, c = 0;
+        for (int g = 0; g < n_seg; ++g) { a += part_gt[g0 + g]; c += part_ge[g0 + g]; }
+        gt[q] = a;
+        ge[q] = c;
+    }
+    if (k == 0) return;
+    if (tid == 0) {
+        int t = 0;
+        for (int g = 0; g < n_seg; ++g) t += cand_n[g0 + g];
+        sh.total = t;
+        sh.cnt = 0;
+    }
+    __syncthreads();
+    const uint64_t* rc = cand + g0 * k;
+    const int* rn = cand_n + g0;
+    auto get = [rc, rn, k](int i) -> uint64_t { return (i % k) < __ldg(rn + i / k) ? __ldg(rc + i) : 0ull; };
+    select_sort_write(get, n_seg * k, sh.total, k, ids + q * k, scores + q * k, sh);
+}
+
+// one CTA per row q: the k best of the R sorted lists ids_in / scores_in [R, Q, k_in] (rank-major, as an all-gather
+// of the per-shard [Q, k_in] results lays them out).  The keys are rebuilt from (score, global id), so the result is
+// the selection over the union of the lists whatever the split; an entry with id < 0 or a non-finite score is dead.
+__global__ void __launch_bounds__(kThreads) topk_cross_merge_kernel(
+    const int64_t* __restrict__ ids_in, const float* __restrict__ scores_in, int R, int64_t Q, int k_in, int k,
+    int64_t* __restrict__ ids, float* __restrict__ scores) {
+    __shared__ MergeShared sh;
+    const int tid = threadIdx.x;
+    const int64_t q = blockIdx.x;
+    auto get = [ids_in, scores_in, Q, k_in, q](int i) -> uint64_t {
+        const int64_t at = (static_cast<int64_t>(i / k_in) * Q + q) * k_in + i % k_in;
+        const int64_t id = __ldg(ids_in + at);
+        const float v = __ldg(scores_in + at);
+        return id >= 0 && finite_score(v) ? cand_key(v, static_cast<uint32_t>(id)) : 0ull;
+    };
+    const int slots = R * k_in;
+    if (tid == 0) { sh.total = 0; sh.cnt = 0; }
+    __syncthreads();
+    int live = 0;
+    for (int i = tid; i < slots; i += kThreads) live += get(i) != 0ull;
+    if (live) atomicAdd(&sh.total, live);
+    __syncthreads();
+    select_sort_write(get, slots, sh.total, k, ids + q * k, scores + q * k, sh);
+}
+
+// row q covers the global columns [col0, col0 + N): a known link c sits at column c - col0
+__global__ void __launch_bounds__(128) score_mask_kernel(float* __restrict__ s, int64_t lds, int64_t N, int64_t col0,
                                                          const int64_t* __restrict__ node,
                                                          const int64_t* __restrict__ rowptr,
                                                          const int32_t* __restrict__ col, int exclude_self) {
@@ -297,11 +340,12 @@ __global__ void __launch_bounds__(128) score_mask_kernel(float* __restrict__ s, 
     if (rowptr != nullptr) {
         const int64_t e1 = rowptr[n + 1];
         for (int64_t e = rowptr[n] + threadIdx.x; e < e1; e += blockDim.x) {
-            const int64_t c = col[e];
+            const int64_t c = col[e] - col0;
             if (c >= 0 && c < N) row[c] = -INFINITY;
         }
     }
-    if (exclude_self && threadIdx.x == 0 && n >= 0 && n < N) row[n] = -INFINITY;
+    const int64_t self = n - col0;
+    if (exclude_self && threadIdx.x == 0 && self >= 0 && self < N) row[self] = -INFINITY;
 }
 
 int64_t n_segments(int64_t N) { return ceil_div(N, kSeg); }
@@ -313,15 +357,21 @@ int64_t align16(int64_t b) { return (b + 15) / 16 * 16; }
 
 using namespace plnlp;
 
-extern "C" int plnlp_score_mask_f32(float* s, int64_t lds, int64_t Q, int64_t N, const int64_t* node,
-                                    const int64_t* rowptr, const int32_t* col, int exclude_self, void* stream) {
-    PLNLP_REQUIRE(Q >= 0 && N >= 1 && lds >= N, PLNLP_E_SIZE);
+extern "C" int plnlp_score_mask_cols_f32(float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0,
+                                         const int64_t* node, const int64_t* rowptr, const int32_t* col,
+                                         int exclude_self, void* stream) {
+    PLNLP_REQUIRE(Q >= 0 && N >= 1 && lds >= N && col0 >= 0 && col0 + N < (int64_t{1} << 31), PLNLP_E_SIZE);
     if (Q == 0) return 0;
     PLNLP_REQUIRE(s && node && (rowptr == nullptr) == (col == nullptr), PLNLP_E_NULL);
     score_mask_kernel<<<static_cast<unsigned>(Q), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-        s, lds, N, node, rowptr, col, exclude_self);
+        s, lds, N, col0, node, rowptr, col, exclude_self);
     PLNLP_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int plnlp_score_mask_f32(float* s, int64_t lds, int64_t Q, int64_t N, const int64_t* node,
+                                    const int64_t* rowptr, const int32_t* col, int exclude_self, void* stream) {
+    return plnlp_score_mask_cols_f32(s, lds, Q, N, 0, node, rowptr, col, exclude_self, stream);
 }
 
 extern "C" int64_t plnlp_topk_rows_workspace_bytes(int64_t Q, int64_t N, int64_t k) {
@@ -330,11 +380,12 @@ extern "C" int64_t plnlp_topk_rows_workspace_bytes(int64_t Q, int64_t N, int64_t
     return align16(slots * k * 8) + 3 * align16(slots * 4);
 }
 
-extern "C" int plnlp_topk_rows_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t k,
-                                   const int64_t* target, const float* target_score, int64_t* ids, float* scores,
-                                   int32_t* gt, int32_t* ge, void* workspace, int64_t workspace_bytes,
-                                   void* stream) {
-    PLNLP_REQUIRE(Q >= 0 && N >= 1 && N < (int64_t{1} << 31) && lds >= N && k >= 0, PLNLP_E_SIZE);
+extern "C" int plnlp_topk_rows_cols_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, int64_t k,
+                                        const int64_t* target, const float* target_score, int64_t* ids,
+                                        float* scores, int32_t* gt, int32_t* ge, void* workspace,
+                                        int64_t workspace_bytes, void* stream) {
+    PLNLP_REQUIRE(Q >= 0 && N >= 1 && lds >= N && k >= 0 && col0 >= 0 && col0 + N < (int64_t{1} << 31),
+                  PLNLP_E_SIZE);
     PLNLP_REQUIRE(k <= kMaxK, PLNLP_E_UNSUPPORTED);
     PLNLP_REQUIRE(k > 0 || target != nullptr, PLNLP_E_SIZE);             // nothing to compute
     if (Q == 0) return 0;
@@ -352,11 +403,33 @@ extern "C" int plnlp_topk_rows_f32(const float* s, int64_t lds, int64_t Q, int64
     int* part_gt = cand_n + align16(slots * 4) / 4;
     int* part_ge = part_gt + align16(slots * 4) / 4;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const float* s_shifted = reinterpret_cast<const float*>(reinterpret_cast<uintptr_t>(s) - 4 * col0);
     topk_segment_kernel<<<static_cast<unsigned>(slots), kThreads, 0, st>>>(
-        s, lds, N, static_cast<int>(k), static_cast<int>(n_seg), target, target_score, cand, cand_n, part_gt, part_ge);
+        s_shifted, lds, col0, col0 + N, static_cast<int>(k), static_cast<int>(n_seg), target, target_score, cand, cand_n, part_gt,
+        part_ge);
     PLNLP_LAUNCH_CHECK();
     topk_merge_kernel<<<static_cast<unsigned>(Q), kThreads, 0, st>>>(
         cand, cand_n, part_gt, part_ge, static_cast<int>(n_seg), static_cast<int>(k), ids, scores, gt, ge);
+    PLNLP_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int plnlp_topk_rows_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t k,
+                                   const int64_t* target, const float* target_score, int64_t* ids, float* scores,
+                                   int32_t* gt, int32_t* ge, void* workspace, int64_t workspace_bytes,
+                                   void* stream) {
+    return plnlp_topk_rows_cols_f32(s, lds, Q, N, 0, k, target, target_score, ids, scores, gt, ge, workspace,
+                                    workspace_bytes, stream);
+}
+
+extern "C" int plnlp_topk_merge_f32(const int64_t* ids_in, const float* scores_in, int64_t R, int64_t Q,
+                                    int64_t k_in, int64_t k, int64_t* ids, float* scores, void* stream) {
+    PLNLP_REQUIRE(R >= 1 && Q >= 0 && k_in >= 1 && k >= 1 && R * k_in < (int64_t{1} << 31), PLNLP_E_SIZE);
+    PLNLP_REQUIRE(k <= kMaxK, PLNLP_E_UNSUPPORTED);
+    if (Q == 0) return 0;
+    PLNLP_REQUIRE(ids_in && scores_in && ids && scores, PLNLP_E_NULL);
+    topk_cross_merge_kernel<<<static_cast<unsigned>(Q), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        ids_in, scores_in, static_cast<int>(R), Q, static_cast<int>(k_in), static_cast<int>(k), ids, scores);
     PLNLP_LAUNCH_CHECK();
     return 0;
 }

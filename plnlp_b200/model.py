@@ -426,14 +426,15 @@ class BaseModel(object):
     def recommend(self, data, nodes, k, exclude=None, exclude_self=True, batch_size=None):
         """extension: the k most likely links of every query node among all nodes -> (ids int64 [Q, k], scores fp32
         [Q, k]) on the device.  ``exclude``: None, 'adj' (the stored rows of data.adj_t) or an int64 [E, 2] edge
-        tensor of known links.  See plnlp_b200/recommend.py."""
+        tensor of known links.  On a row-partitioned model a collective call (every rank, same arguments, full result
+        everywhere).  See plnlp_b200/recommend.py."""
         from . import recommend
         return recommend.recommend(self, data, nodes, k, exclude, exclude_self, batch_size)
 
     def rank_against_all(self, data, edges, exclude=None, exclude_self=True, batch_size=None):
         """extension: filtered full-ranking evaluation -> fp32 [P], the rank of every target among all nodes for
         its source (1 + (gt + ge) / 2; known links other than the target itself filtered out).  Feed it to
-        utils.full_rank_metrics.  See plnlp_b200/recommend.py."""
+        utils.full_rank_metrics.  On a row-partitioned model a collective call.  See plnlp_b200/recommend.py."""
         from . import recommend
         return recommend.rank_against_all(self, data, edges, exclude, exclude_self, batch_size)
 
