@@ -371,6 +371,18 @@ int plnlp_topk_rows_cols_f32(const float* s, int64_t lds, int64_t Q, int64_t N, 
                              const int64_t* target, const float* target_score,
                              int64_t* ids, float* scores, int32_t* gt, int32_t* ge,
                              void* workspace, int64_t workspace_bytes, void* stream);
+/* Candidate-set forms: s [Q, C] holds the candidates cand[0 .. C), strictly ascending global node ids (the caller's
+ * promise).  The mask finds each known link and node[q] by binary search in cand and skips an id that is not there.
+ * The select keeps its keys on the column, which orders as the ids do, and reports ids cand[j]; target[q] is a global
+ * id, compared with the column it occupies (none when it is not in cand, and then every column counts).
+ * cand == NULL in plnlp_topk_rows_cand_f32 is plnlp_topk_rows_cols_f32; with cand, col0 must be 0
+ * (PLNLP_E_UNSUPPORTED).  Workspace as plnlp_topk_rows_cols_f32. */
+int plnlp_score_mask_cand_f32(float* s, int64_t lds, int64_t Q, int64_t C, const int64_t* cand, const int64_t* node,
+                              const int64_t* rowptr, const int32_t* col, int exclude_self, void* stream);
+int plnlp_topk_rows_cand_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, int64_t k,
+                             const int64_t* target, const float* target_score,
+                             int64_t* ids, float* scores, int32_t* gt, int32_t* ge,
+                             void* workspace, int64_t workspace_bytes, const int64_t* cand, void* stream);
 /* Cross-shard merge: ids_in / scores_in [R, Q, k_in] (rank-major: the all-gather of R per-shard [Q, k_in] results)
  * -> ids / scores [Q, k] (1 <= k <= 1024): per row the k best entries of the R lists by score descending then id
  * ascending, the tail (-1, -inf).  An entry with id < 0 or a non-finite score is dead.  Keys are rebuilt from

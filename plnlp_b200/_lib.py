@@ -64,6 +64,8 @@ SIGNATURES = {
     "plnlp_topk_rows_f32": (c_int, [_P, _L, _L, _L, _L, _P, _P, _P, _P, _P, _P, _P, _L, _P]),
     "plnlp_score_mask_cols_f32": (c_int, [_P, _L, _L, _L, _L, _P, _P, _P, _I, _P]),
     "plnlp_topk_rows_cols_f32": (c_int, [_P, _L, _L, _L, _L, _L, _P, _P, _P, _P, _P, _P, _P, _L, _P]),
+    "plnlp_score_mask_cand_f32": (c_int, [_P, _L, _L, _L, _P, _P, _P, _P, _I, _P]),
+    "plnlp_topk_rows_cand_f32": (c_int, [_P, _L, _L, _L, _L, _L, _P, _P, _P, _P, _P, _P, _P, _L, _P, _P]),
     "plnlp_topk_merge_f32": (c_int, [_P, _P, _L, _L, _L, _L, _P, _P, _P]),
     "plnlp_graph_make_keys": (c_int, [_P, _P, _L, _L, _I, _I, _P, _P, _P]),
     "plnlp_graph_diag_keys": (c_int, [_L, _L, _P, _P, _L, _P]),

@@ -1142,10 +1142,16 @@ def mrr_counts_raw(pos, neg):
     return gt, ge
 
 
-def score_mask_raw(s, nodes, rowptr=None, col=None, exclude_self=True, col0=0):
+def _cand_ids(cand, N):
+    if cand.dtype != torch.int64 or cand.dim() != 1 or cand.numel() != N:
+        raise RuntimeError("cand must be int64 with one entry per score column")
+    return cand.contiguous()
+
+
+def score_mask_raw(s, nodes, rowptr=None, col=None, exclude_self=True, col0=0, cand=None):
     """in place: s[q, j] = -inf for the known links j of nodes[q] (CSR rowptr int64 / col int32) and, with
     ``exclude_self``, for j = nodes[q].  The chunk covers the global candidate ids [col0, col0 + N): col and nodes
-    are global ids."""
+    are global ids.  ``cand`` (int64 [N], strictly ascending global ids): column j is the node cand[j] instead."""
     lib = _lib.load()
     if _f32c(s).dim() != 2 or s.stride(1) != 1:
         raise RuntimeError("the score chunk must be a 2-D fp32 matrix with unit column stride (masked in place)")
@@ -1157,17 +1163,24 @@ def score_mask_raw(s, nodes, rowptr=None, col=None, exclude_self=True, col0=0):
     if col is not None and (rowptr.dtype != torch.int64 or col.dtype != torch.int32):
         raise RuntimeError("the known-link CSR is int64 rowptr + int32 col")
     Q, N = s.shape
+    if cand is not None:
+        cand = _cand_ids(cand, N)
+        with profiling.span("score_mask_f32", 0, 0):
+            check(lib.plnlp_score_mask_cand_f32(ptr(s), _ld(s), Q, N, ptr(cand), ptr(nodes), ptr(rowptr), ptr(col),
+                                                int(bool(exclude_self)), stream()), "plnlp_score_mask_cand_f32")
+        return s
     with profiling.span("score_mask_f32", 0, 0):
         check(lib.plnlp_score_mask_cols_f32(ptr(s), _ld(s), Q, N, int(col0), ptr(nodes), ptr(rowptr), ptr(col),
                                             int(bool(exclude_self)), stream()), "plnlp_score_mask_cols_f32")
     return s
 
 
-def topk_rows_raw(s, k, target=None, target_score=None, col0=0):
+def topk_rows_raw(s, k, target=None, target_score=None, col0=0, cand=None):
     """per row of s [Q, N]: the k largest finite entries (score descending, then column ascending; tail (-1, -inf))
     and, with ``target``, the filtered rank counts gt / ge against ``target_score``.  -> (ids int64 [Q, k] or None,
     scores [Q, k] or None, gt int32 [Q] or None, ge int32 [Q] or None).  One read of s.  The chunk covers the
-    global candidate ids [col0, col0 + N): ids, ties and ``target`` are global ids."""
+    global candidate ids [col0, col0 + N): ids, ties and ``target`` are global ids.  ``cand`` (int64 [N], strictly
+    ascending global ids, col0 = 0): column j is the node cand[j]; ids are cand[j], ``target`` stays a global id."""
     lib = _lib.load()
     s = _rowmajor(s)
     Q, N = s.shape
@@ -1184,6 +1197,13 @@ def topk_rows_raw(s, k, target=None, target_score=None, col0=0):
         ge = torch.empty(Q, dtype=torch.int32, device=dev)
     nbytes = max(int(lib.plnlp_topk_rows_workspace_bytes(Q, N, max(int(k), 0))), 16)
     ws = workspace.get("topk_rows", nbytes, dev)
+    if cand is not None:
+        cand = _cand_ids(cand, N)
+        with profiling.span(f"topk_rows_f32 k={k}", Q * N * 4, 0):
+            check(lib.plnlp_topk_rows_cand_f32(ptr(s), _ld(s), Q, N, int(col0), int(k), ptr(target),
+                                               ptr(target_score), ptr(ids), ptr(scores), ptr(gt), ptr(ge), ptr(ws),
+                                               nbytes, ptr(cand), stream()), "plnlp_topk_rows_cand_f32")
+        return ids, scores, gt, ge
     with profiling.span(f"topk_rows_f32 k={k}", Q * N * 4, 0):
         check(lib.plnlp_topk_rows_cols_f32(ptr(s), _ld(s), Q, N, int(col0), int(k), ptr(target), ptr(target_score),
                                            ptr(ids), ptr(scores), ptr(gt), ptr(ge), ptr(ws), nbytes, stream()),

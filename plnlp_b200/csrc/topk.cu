@@ -10,6 +10,10 @@
 // graph): keys, ids and the target comparison then use the global column col0 + j, so per-shard results merge
 // into exactly the selection over the whole row (topk_cross_merge_kernel).
 //
+// A chunk may instead hold an arbitrary candidate set: column j is the node cand[j], cand strictly ascending.  Keys
+// stay on the column, which orders exactly as the ids do; the mask and the target comparison find a node's column by
+// binary search in cand, and the write tail reports cand[j].
+//
 // Two kernels, ONE pass over the score chunk:
 //   topk_segment_kernel  one CTA per (row, segment of kSeg columns).  Streams its segment once, counts gt / ge
 //                        against the target score, and keeps a candidate buffer in shared memory: an entry is
@@ -38,6 +42,16 @@ constexpr int64_t kSeg = 65536;                    // columns per segment CTA
 static_assert(kCap >= kMaxK + kTile, "a tile must fit behind k kept candidates");
 
 __device__ __forceinline__ bool finite_score(float v) { return fabsf(v) <= FLT_MAX; }
+
+// the column of node id among the strictly ascending cand[c0 .. c1), or -1
+__device__ __forceinline__ int64_t cand_column(const int64_t* __restrict__ cand, int64_t c0, int64_t c1, int64_t id) {
+    int64_t lo = c0, hi = c1;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(cand + mid) < id) lo = mid + 1; else hi = mid;
+    }
+    return lo < c1 && __ldg(cand + lo) == id ? lo : -1;
+}
 
 __device__ __forceinline__ uint64_t cand_key(float v, uint32_t col) {
     const float c = v == 0.0f ? 0.0f : v;          // -0 ties with +0
@@ -151,11 +165,14 @@ __device__ void cut_to_k(SegShared& sh, int k) {
 
 // grid.x = Q * n_seg; CTA b handles row b / n_seg, global columns [col0 + seg * kSeg, min(col_end, ... + kSeg)).
 // s_shifted = s - col0 (formed as an address by the host), so the loop runs on global columns: the column offset
-// costs no register (the kernel stays at 62 registers, 4 CTAs per SM).
+// costs no register (the kernel stays at 62 registers, 4 CTAs per SM).  kIdCols (then col0 = 0): column j is the
+// node col_id[j], and the target's column is looked up once, before the loop, within this CTA's segment -- a
+// separate instantiation, so the lookup leaves the plain kernel's code and register allocation as they were.
+template <bool kIdCols>
 __global__ void __launch_bounds__(kThreads, 4) topk_segment_kernel(
     const float* __restrict__ s_shifted, int64_t lds, int64_t col0, int64_t col_end, int k, int n_seg,
-    const int64_t* __restrict__ target, const float* __restrict__ target_score, uint64_t* __restrict__ cand,
-    int* __restrict__ cand_n, int* __restrict__ part_gt, int* __restrict__ part_ge) {
+    const int64_t* __restrict__ target, const float* __restrict__ target_score, const int64_t* __restrict__ col_id,
+    uint64_t* __restrict__ cand, int* __restrict__ cand_n, int* __restrict__ part_gt, int* __restrict__ part_ge) {
     __shared__ SegShared sh;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t b = blockIdx.x;
@@ -163,7 +180,8 @@ __global__ void __launch_bounds__(kThreads, 4) topk_segment_kernel(
     const int64_t c0 = col0 + (b % n_seg) * kSeg, c1 = min(col_end, c0 + kSeg);
     const float* row = s_shifted + q * lds;
     const bool rank = target != nullptr;
-    const int64_t tcol = rank ? target[q] : -1;
+    int64_t tcol = rank ? target[q] : -1;
+    if constexpr (kIdCols) tcol = rank ? cand_column(col_id, c0, c1, tcol) : -1;
     const float tval = rank ? target_score[q] : 0.0f;
     int cgt = 0, cge = 0;
     if (tid == 0) { sh.cnt = 0; sh.thr = 0ull; }   // every finite entry has a key > 0
@@ -234,10 +252,10 @@ struct MergeShared {
 
 // the tail of both merges, run by one CTA for one row: the k best of the keys get(0 .. slots) -- ``total`` of them
 // live, dead slots read as key 0, below every live key -- sorted descending (bitonic, shared memory) and written as
-// (id, score), the tail (-1, -inf).  Begins in sync.
+// (id, score), the tail (-1, -inf); id = col_id[column] when col_id != NULL.  Begins in sync.
 template <class Get>
-__device__ void select_sort_write(Get get, int slots, int total, int k, int64_t* __restrict__ ids,
-                                  float* __restrict__ scores, MergeShared& sh) {
+__device__ void select_sort_write(Get get, int slots, int total, int k, const int64_t* __restrict__ col_id,
+                                  int64_t* __restrict__ ids, float* __restrict__ scores, MergeShared& sh) {
     const int tid = threadIdx.x;
     const int m = min(total, k);
     const uint64_t kth = total > k ? block_select(get, slots, k, sh.sel) : 1ull;
@@ -265,7 +283,8 @@ __device__ void select_sort_write(Get get, int slots, int total, int k, int64_t*
     for (int i = tid; i < k; i += kThreads) {
         if (i < m) {
             const uint64_t key = sh.buf[i];
-            ids[i] = static_cast<int64_t>(~static_cast<uint32_t>(key));
+            const uint32_t c = ~static_cast<uint32_t>(key);
+            ids[i] = col_id != nullptr ? __ldg(col_id + c) : static_cast<int64_t>(c);
             scores[i] = key_float(static_cast<uint32_t>(key >> 32));
         } else {
             ids[i] = -1;
@@ -275,11 +294,11 @@ __device__ void select_sort_write(Get get, int slots, int total, int k, int64_t*
 }
 
 // one CTA per row: gt / ge sums, then the k best of the n_seg * k candidate slots (slot i of segment g is live when
-// i < cand_n[g]), sorted, written as (id, score)
+// i < cand_n[g]), sorted, written as (id, score); the id of column j is col_id[j] when col_id != NULL
 __global__ void __launch_bounds__(kThreads) topk_merge_kernel(
     const uint64_t* __restrict__ cand, const int* __restrict__ cand_n, const int* __restrict__ part_gt,
-    const int* __restrict__ part_ge, int n_seg, int k, int64_t* __restrict__ ids, float* __restrict__ scores,
-    int32_t* __restrict__ gt, int32_t* __restrict__ ge) {
+    const int* __restrict__ part_ge, int n_seg, int k, const int64_t* __restrict__ col_id, int64_t* __restrict__ ids,
+    float* __restrict__ scores, int32_t* __restrict__ gt, int32_t* __restrict__ ge) {
     __shared__ MergeShared sh;
     const int tid = threadIdx.x;
     const int64_t q = blockIdx.x;
@@ -301,7 +320,7 @@ __global__ void __launch_bounds__(kThreads) topk_merge_kernel(
     const uint64_t* rc = cand + g0 * k;
     const int* rn = cand_n + g0;
     auto get = [rc, rn, k](int i) -> uint64_t { return (i % k) < __ldg(rn + i / k) ? __ldg(rc + i) : 0ull; };
-    select_sort_write(get, n_seg * k, sh.total, k, ids + q * k, scores + q * k, sh);
+    select_sort_write(get, n_seg * k, sh.total, k, col_id, ids + q * k, scores + q * k, sh);
 }
 
 // one CTA per row q: the k best of the R sorted lists ids_in / scores_in [R, Q, k_in] (rank-major, as an all-gather
@@ -326,11 +345,13 @@ __global__ void __launch_bounds__(kThreads) topk_cross_merge_kernel(
     for (int i = tid; i < slots; i += kThreads) live += get(i) != 0ull;
     if (live) atomicAdd(&sh.total, live);
     __syncthreads();
-    select_sort_write(get, slots, sh.total, k, ids + q * k, scores + q * k, sh);
+    select_sort_write(get, slots, sh.total, k, nullptr, ids + q * k, scores + q * k, sh);
 }
 
-// row q covers the global columns [col0, col0 + N): a known link c sits at column c - col0
+// row q covers the global columns [col0, col0 + N): a known link c sits at column c - col0; or, with cand (col0 = 0),
+// the nodes cand[0 .. N): c sits at its position in cand, if any
 __global__ void __launch_bounds__(128) score_mask_kernel(float* __restrict__ s, int64_t lds, int64_t N, int64_t col0,
+                                                         const int64_t* __restrict__ cand,
                                                          const int64_t* __restrict__ node,
                                                          const int64_t* __restrict__ rowptr,
                                                          const int32_t* __restrict__ col, int exclude_self) {
@@ -340,11 +361,11 @@ __global__ void __launch_bounds__(128) score_mask_kernel(float* __restrict__ s, 
     if (rowptr != nullptr) {
         const int64_t e1 = rowptr[n + 1];
         for (int64_t e = rowptr[n] + threadIdx.x; e < e1; e += blockDim.x) {
-            const int64_t c = col[e] - col0;
+            const int64_t c = cand != nullptr ? cand_column(cand, 0, N, col[e]) : col[e] - col0;
             if (c >= 0 && c < N) row[c] = -INFINITY;
         }
     }
-    const int64_t self = n - col0;
+    const int64_t self = cand != nullptr ? (exclude_self ? cand_column(cand, 0, N, n) : -1) : n - col0;
     if (exclude_self && threadIdx.x == 0 && self >= 0 && self < N) row[self] = -INFINITY;
 }
 
@@ -357,16 +378,32 @@ int64_t align16(int64_t b) { return (b + 15) / 16 * 16; }
 
 using namespace plnlp;
 
-extern "C" int plnlp_score_mask_cols_f32(float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0,
-                                         const int64_t* node, const int64_t* rowptr, const int32_t* col,
-                                         int exclude_self, void* stream) {
+namespace {
+
+int score_mask(float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, const int64_t* cand, const int64_t* node,
+               const int64_t* rowptr, const int32_t* col, int exclude_self, void* stream) {
     PLNLP_REQUIRE(Q >= 0 && N >= 1 && lds >= N && col0 >= 0 && col0 + N < (int64_t{1} << 31), PLNLP_E_SIZE);
     if (Q == 0) return 0;
     PLNLP_REQUIRE(s && node && (rowptr == nullptr) == (col == nullptr), PLNLP_E_NULL);
     score_mask_kernel<<<static_cast<unsigned>(Q), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-        s, lds, N, col0, node, rowptr, col, exclude_self);
+        s, lds, N, col0, cand, node, rowptr, col, exclude_self);
     PLNLP_LAUNCH_CHECK();
     return 0;
+}
+
+}  // namespace
+
+extern "C" int plnlp_score_mask_cols_f32(float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0,
+                                         const int64_t* node, const int64_t* rowptr, const int32_t* col,
+                                         int exclude_self, void* stream) {
+    return score_mask(s, lds, Q, N, col0, nullptr, node, rowptr, col, exclude_self, stream);
+}
+
+extern "C" int plnlp_score_mask_cand_f32(float* s, int64_t lds, int64_t Q, int64_t C, const int64_t* cand,
+                                         const int64_t* node, const int64_t* rowptr, const int32_t* col,
+                                         int exclude_self, void* stream) {
+    PLNLP_REQUIRE(Q == 0 || cand, PLNLP_E_NULL);
+    return score_mask(s, lds, Q, C, 0, cand, node, rowptr, col, exclude_self, stream);
 }
 
 extern "C" int plnlp_score_mask_f32(float* s, int64_t lds, int64_t Q, int64_t N, const int64_t* node,
@@ -380,13 +417,13 @@ extern "C" int64_t plnlp_topk_rows_workspace_bytes(int64_t Q, int64_t N, int64_t
     return align16(slots * k * 8) + 3 * align16(slots * 4);
 }
 
-extern "C" int plnlp_topk_rows_cols_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, int64_t k,
+extern "C" int plnlp_topk_rows_cand_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, int64_t k,
                                         const int64_t* target, const float* target_score, int64_t* ids,
                                         float* scores, int32_t* gt, int32_t* ge, void* workspace,
-                                        int64_t workspace_bytes, void* stream) {
+                                        int64_t workspace_bytes, const int64_t* cand, void* stream) {
     PLNLP_REQUIRE(Q >= 0 && N >= 1 && lds >= N && k >= 0 && col0 >= 0 && col0 + N < (int64_t{1} << 31),
                   PLNLP_E_SIZE);
-    PLNLP_REQUIRE(k <= kMaxK, PLNLP_E_UNSUPPORTED);
+    PLNLP_REQUIRE(k <= kMaxK && (cand == nullptr || col0 == 0), PLNLP_E_UNSUPPORTED);
     PLNLP_REQUIRE(k > 0 || target != nullptr, PLNLP_E_SIZE);             // nothing to compute
     if (Q == 0) return 0;
     PLNLP_REQUIRE(s && workspace, PLNLP_E_NULL);
@@ -398,20 +435,29 @@ extern "C" int plnlp_topk_rows_cols_f32(const float* s, int64_t lds, int64_t Q, 
     const int64_t slots = Q * n_seg;
     PLNLP_REQUIRE(slots < (int64_t{1} << 31), PLNLP_E_SIZE);
     char* w = static_cast<char*>(workspace);
-    uint64_t* cand = reinterpret_cast<uint64_t*>(w);
+    uint64_t* keys = reinterpret_cast<uint64_t*>(w);
     int* cand_n = reinterpret_cast<int*>(w + align16(slots * k * 8));
     int* part_gt = cand_n + align16(slots * 4) / 4;
     int* part_ge = part_gt + align16(slots * 4) / 4;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const float* s_shifted = reinterpret_cast<const float*>(reinterpret_cast<uintptr_t>(s) - 4 * col0);
-    topk_segment_kernel<<<static_cast<unsigned>(slots), kThreads, 0, st>>>(
-        s_shifted, lds, col0, col0 + N, static_cast<int>(k), static_cast<int>(n_seg), target, target_score, cand, cand_n, part_gt,
-        part_ge);
+    auto segment = cand != nullptr ? topk_segment_kernel<true> : topk_segment_kernel<false>;
+    segment<<<static_cast<unsigned>(slots), kThreads, 0, st>>>(
+        s_shifted, lds, col0, col0 + N, static_cast<int>(k), static_cast<int>(n_seg), target, target_score, cand,
+        keys, cand_n, part_gt, part_ge);
     PLNLP_LAUNCH_CHECK();
     topk_merge_kernel<<<static_cast<unsigned>(Q), kThreads, 0, st>>>(
-        cand, cand_n, part_gt, part_ge, static_cast<int>(n_seg), static_cast<int>(k), ids, scores, gt, ge);
+        keys, cand_n, part_gt, part_ge, static_cast<int>(n_seg), static_cast<int>(k), cand, ids, scores, gt, ge);
     PLNLP_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int plnlp_topk_rows_cols_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t col0, int64_t k,
+                                        const int64_t* target, const float* target_score, int64_t* ids,
+                                        float* scores, int32_t* gt, int32_t* ge, void* workspace,
+                                        int64_t workspace_bytes, void* stream) {
+    return plnlp_topk_rows_cand_f32(s, lds, Q, N, col0, k, target, target_score, ids, scores, gt, ge, workspace,
+                                    workspace_bytes, nullptr, stream);
 }
 
 extern "C" int plnlp_topk_rows_f32(const float* s, int64_t lds, int64_t Q, int64_t N, int64_t k,

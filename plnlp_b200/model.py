@@ -423,20 +423,22 @@ class BaseModel(object):
             return evaluate_hits(evaluator, pos_valid_pred, neg_valid_pred, pos_test_pred, neg_test_pred)
         return evaluate_mrr(evaluator, pos_valid_pred, neg_valid_pred, pos_test_pred, neg_test_pred)
 
-    def recommend(self, data, nodes, k, exclude=None, exclude_self=True, batch_size=None):
+    def recommend(self, data, nodes, k, exclude=None, exclude_self=True, batch_size=None, candidates=None):
         """extension: the k most likely links of every query node among all nodes -> (ids int64 [Q, k], scores fp32
         [Q, k]) on the device.  ``exclude``: None, 'adj' (the stored rows of data.adj_t) or an int64 [E, 2] edge
-        tensor of known links.  On a row-partitioned model a collective call (every rank, same arguments, full result
-        everywhere).  See plnlp_b200/recommend.py."""
+        tensor of known links.  ``candidates``: an int64 tensor of node ids; only those are recommended.  On a
+        row-partitioned model a collective call (every rank, same arguments, full result everywhere).  See
+        plnlp_b200/recommend.py."""
         from . import recommend
-        return recommend.recommend(self, data, nodes, k, exclude, exclude_self, batch_size)
+        return recommend.recommend(self, data, nodes, k, exclude, exclude_self, batch_size, candidates)
 
-    def rank_against_all(self, data, edges, exclude=None, exclude_self=True, batch_size=None):
+    def rank_against_all(self, data, edges, exclude=None, exclude_self=True, batch_size=None, candidates=None):
         """extension: filtered full-ranking evaluation -> fp32 [P], the rank of every target among all nodes for
-        its source (1 + (gt + ge) / 2; known links other than the target itself filtered out).  Feed it to
-        utils.full_rank_metrics.  On a row-partitioned model a collective call.  See plnlp_b200/recommend.py."""
+        its source (1 + (gt + ge) / 2; known links other than the target itself filtered out).  ``candidates``: rank
+        among those node ids and the target instead.  Feed it to utils.full_rank_metrics.  On a row-partitioned model
+        a collective call.  See plnlp_b200/recommend.py."""
         from . import recommend
-        return recommend.rank_against_all(self, data, edges, exclude, exclude_self, batch_size)
+        return recommend.rank_against_all(self, data, edges, exclude, exclude_self, batch_size, candidates)
 
 
 def create_input_layer(num_nodes, num_node_feats, hidden_channels, use_node_feats=True,

@@ -1,13 +1,16 @@
 """Time link recommendation over all nodes (BaseModel.recommend / rank_against_all) at the BASELINE graph shapes.
 
-Usage: python tools/recommend_bench.py [citation2|ddi|collab] --predictor DOT|MLP --queries Q --k K [--out FILE]
+Usage: python tools/recommend_bench.py [citation2|ddi|collab] --predictor DOT|MLP --queries Q --k K
+       [--candidates COUNT] [--out FILE]
 
 Prints one JSON line: ms per query and candidate pairs/s of both calls (timed with CUDA events after a warm-up, the
 profiler off), then the per-kernel split of one instrumented ``recommend`` call (plnlp_b200.profiling spans): the
 score GEMM's TFLOP/s and the select kernel's GB/s and share of the HBM copy peak (bytes = passes x Q x N x 4; the
 select reads each score row once).  The card's name and power limit come from a read-only nvidia-smi query.  With the
 MLP head at citation2 shape every query costs 2 H H1 FLOP per candidate: the run times the given sample of queries and
-the all-nodes figure is an extrapolation, labelled as such."""
+the all-nodes figure is an extrapolation, labelled as such.  ``--candidates COUNT`` restricts both calls to COUNT
+distinct random nodes (seeded): pairs, GEMM width and select bytes then count |C| candidates per query, and the line
+gains a "candidates" field."""
 import argparse
 import json
 import os
@@ -56,6 +59,7 @@ def main():
     ap.add_argument("--k", type=int, default=100)
     ap.add_argument("--exclude", default="adj", choices=["adj", "none"])
     ap.add_argument("--reps", type=int, default=2)
+    ap.add_argument("--candidates", type=int, default=None, help="restrict to this many random nodes")
     ap.add_argument("--out", default=None, help="also append the JSON line to this file")
     a = ap.parse_args()
 
@@ -69,9 +73,13 @@ def main():
     g = torch.Generator(device=dev).manual_seed(3)
     nodes = torch.randint(0, N, (Q,), generator=g, device=dev)
     edges = torch.stack([nodes, torch.randint(0, N, (Q,), generator=g, device=dev)], 1)
+    cand, W = None, N
+    if a.candidates is not None:
+        cand = torch.randperm(N, generator=g, device=dev)[:a.candidates]
+        W = cand.numel()
 
-    rec = lambda: model.recommend(data, nodes, a.k, exclude=exclude)          # noqa: E731
-    rank = lambda: model.rank_against_all(data, edges, exclude=exclude)      # noqa: E731
+    rec = lambda: model.recommend(data, nodes, a.k, exclude=exclude, candidates=cand)          # noqa: E731
+    rank = lambda: model.rank_against_all(data, edges, exclude=exclude, candidates=cand)      # noqa: E731
     rec()                                                                    # warm-up: every shape the timing uses
     rank()
     enc_ms, _ = timed(lambda: model.encode_for_test(data), a.reps)
@@ -86,7 +94,7 @@ def main():
     other = {}
     for name, s in spans.items():
         if name.startswith("gemm") or name.startswith("edge_mlp_fwd_fused"):
-            if "x{}x".format(N) in name or name.startswith("edge_mlp_fwd_fused"):   # the score chunks, not the encoder
+            if "x{}x".format(W) in name or name.startswith("edge_mlp_fwd_fused"):   # the score chunks, not the encoder
                 gemm["ms"] += s["ms"]
                 gemm["flops"] += s["flops"]
                 continue
@@ -95,15 +103,15 @@ def main():
             select["n"] += s["n"]
             continue
         other[name] = round(s["ms"], 3)
-    sel_bytes = SELECT_PASSES * Q * N * 4
+    sel_bytes = SELECT_PASSES * Q * W * 4
     res = {
         "workload": cfg["name"], "N": N, "predictor": a.predictor, "queries": Q, "k": a.k, "exclude": a.exclude,
         "gpu": gpu_info(),
         "encode_ms": round(enc_ms, 3),
         "recommend": {"ms": round(rec_ms, 3), "ms_per_query": round(rec_ms / Q, 5),
-                      "pairs_per_s": round(Q * N / rec_ms * 1e3)},
+                      "pairs_per_s": round(Q * W / rec_ms * 1e3)},
         "rank_against_all": {"ms": round(rank_ms, 3), "ms_per_query": round(rank_ms / Q, 5),
-                             "pairs_per_s": round(Q * N / rank_ms * 1e3),
+                             "pairs_per_s": round(Q * W / rank_ms * 1e3),
                              "metrics_random_targets": {k: round(v, 6) for k, v in full_rank_metrics(ranks).items()}},
         "split_one_recommend_call": {
             "score_ms": round(gemm["ms"], 3), "score_ms_per_query": round(gemm["ms"] / Q, 5),
@@ -117,6 +125,8 @@ def main():
                                      "note": f"extrapolated from {Q} timed queries to all {N} nodes"},
         "valid_ids_first_row": int((ids[0] >= 0).sum()),
     }
+    if cand is not None:
+        res["candidates"] = W
     line = json.dumps(res)
     print(line)
     if a.out:

@@ -1,13 +1,16 @@
 """Time candidate-sharded link recommendation (BaseModel.recommend / rank_against_all on a row-partitioned model) at
 the citation2 shape, built and partitioned the way bench.measure does it.
 
-Usage: torchrun --nproc_per_node R tools/recommend_partitioned_bench.py [--runs DOT:100:1000,MLP:100:20] [--out FILE]
+Usage: torchrun --nproc_per_node R tools/recommend_partitioned_bench.py [--runs DOT:100:1000,MLP:100:20]
+       [--candidates COUNT] [--out FILE]
 (without torchrun: one rank, a one-rank NCCL group)
 
 Prints one JSON line per run from rank 0: the card's name and power limit, ms per query of both calls (CUDA events
 around calls that end in a device synchronise, after a warm-up, the profiler off), and per rank the split of one
 instrumented ``recommend`` call (plnlp_b200.profiling spans): score GEMM / fused MLP (ms, TFLOP/s), mask + select,
-exclusion build, exchange (query rows, all-gather of the top-k lists) and merge, encode of the row block."""
+exclusion build, exchange (query rows, all-gather of the top-k lists) and merge, encode of the row block.
+``--candidates COUNT`` restricts every run to COUNT distinct random nodes (the same on every rank); the lines then
+gain a "candidates" field."""
 import argparse
 import json
 import os
@@ -20,7 +23,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.dont_write_bytecode = True
 import bench  # noqa: E402
-from plnlp_b200 import parallel, profiling  # noqa: E402
+from plnlp_b200 import parallel, profiling, recommend  # noqa: E402
 from plnlp_b200.graph import CSRGraph  # noqa: E402
 from plnlp_b200.utils import gcn_normalization  # noqa: E402
 from tools.recommend_bench import gpu_info, timed  # noqa: E402
@@ -56,6 +59,7 @@ def main():
                     help="comma-separated PREDICTOR:K:QUERIES")
     ap.add_argument("--exclude", default="adj", choices=["adj", "none"])
     ap.add_argument("--reps", type=int, default=2)
+    ap.add_argument("--candidates", type=int, default=None, help="restrict to this many random nodes")
     ap.add_argument("--out", default=None, help="also append the JSON lines to this file (rank 0)")
     a = ap.parse_args()
 
@@ -85,8 +89,13 @@ def main():
             g = torch.Generator(device=dev).manual_seed(3)       # the same queries on every rank
             nodes = torch.randint(0, N, (Q,), generator=g, device=dev)
             edges = torch.stack([nodes, torch.randint(0, N, (Q,), generator=g, device=dev)], 1)
-            rec = lambda: model.recommend(data, nodes, k, exclude=exclude)          # noqa: E731
-            rnk = lambda: model.rank_against_all(data, edges, exclude=exclude)      # noqa: E731
+            cand, width = None, hi - lo
+            if a.candidates is not None:
+                cand = torch.unique(torch.randperm(N, generator=g, device=dev)[:a.candidates])
+                x, y = recommend.candidate_slices(cand, [(lo, hi)])[0]
+                width = y - x
+            rec = lambda: model.recommend(data, nodes, k, exclude=exclude, candidates=cand)          # noqa: E731
+            rnk = lambda: model.rank_against_all(data, edges, exclude=exclude, candidates=cand)      # noqa: E731
             rec()                                                                    # warm-up
             rnk()
             dist.barrier()
@@ -95,7 +104,7 @@ def main():
             rank_ms, _ = timed(rnk, a.reps)
             profiling.enable()
             rec()
-            split = split_of(profiling.disable(), hi - lo)
+            split = split_of(profiling.disable(), width)
             splits = [None] * world
             dist.all_gather_object(splits, split)
             times = torch.tensor([rec_ms, rank_ms], dtype=torch.float64, device=dev)
@@ -109,6 +118,8 @@ def main():
                        "timing": f"CUDA events on rank 0 around {a.reps} calls, max over ranks",
                        "split_one_recommend_call_per_rank": splits,
                        "valid_ids_first_row": int((ids[0] >= 0).sum())}
+                if cand is not None:
+                    res["candidates"] = cand.numel()
                 line = json.dumps(res)
                 print(line, flush=True)
                 if a.out:
