@@ -234,6 +234,16 @@ int plnlp_segment_softmax_fwd_f32(const int64_t* rowptr, int64_t n_rows, const f
                                   void* stream);
 int plnlp_segment_softmax_bwd_f32(const int64_t* rowptr, int64_t n_rows, const float* alpha, const float* dalpha,
                                   float scale, float* ds, void* stream);
+/* Attention scores of a CSR row block against separate query and key tables: score[e] = <q[row(e)], k[col(e)]> for
+ * every stored entry e, written in CSR entry order.  The block is walked through its SpMM work plan (item_ptr has
+ * n_items + 1 offsets into col; item i holds the entries [item_ptr[i], item_ptr[i+1]) of row item_row[i]; graph.py
+ * build_plan), so hub rows are split across warps.  q is [n_q, F] with leading dimension ldq, k is [n_k, F] with ldk.
+ * Each score is bit-identical to plnlp_edge_dot_fwd_f32 over the pairs (row, n_q + col) of the stacked table [q; k].
+ * Serves the row-partitioned TransformerConv (layer.py, _ops.BlockAttention): forward s = score(q, k) and backward
+ * dalpha = score(g, v). */
+int plnlp_attn_score_csr_f32(const int32_t* item_ptr, const int32_t* item_row, int64_t n_items, const int32_t* col,
+                             const float* q, int64_t ldq, const float* k, int64_t ldk, int64_t F, float* score,
+                             void* stream);
 
 /* Plain endpoint gather out[p, :] = h[idx[p * idx_stride], :] (negative indices wrap) and its backward
  * grad_h[n, :] = sum_{t in segment n} g[entry[t], :] over a node-sorted entry list (seg_ptr has n_seg + 1

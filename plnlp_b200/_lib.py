@@ -38,6 +38,7 @@ SIGNATURES = {
     "plnlp_gather_hadamard_f32": (c_int, [_P, _L, _L, _P, _L, _L, _P, _L, _P]),
     "plnlp_segment_softmax_fwd_f32": (c_int, [_P, _L, _P, _F, _P, _P]),
     "plnlp_segment_softmax_bwd_f32": (c_int, [_P, _L, _P, _P, _F, _P, _P]),
+    "plnlp_attn_score_csr_f32": (c_int, [_P, _P, _L, _P, _P, _L, _P, _L, _L, _P, _P]),
     "plnlp_gather_rows_f32": (c_int, [_P, _L, _L, _P, _L, _L, _L, _P, _L, _P]),
     "plnlp_row_scatter_sorted_f32": (c_int, [_P, _L, _L, _P, _L, _P, _P, _L, _P]),
     "plnlp_edge_dot_fwd_f32": (c_int, [_P, _L, _L, _P, _L, _L, _P, _P]),

@@ -649,12 +649,14 @@ class FusedLinear(torch.autograd.Function):
     intermediate.  W_i may be a column slice of a larger weight (leading dimension respected)."""
 
     @staticmethod
-    def forward(ctx, bias, act, drop_p, seed, n, *xw):
+    def forward(ctx, bias, addend, act, drop_p, seed, n, *xw):
         xs, ws = xw[:n], xw[n:]
-        Y = None
+        # ``addend`` (optional): accumulated in the first GEMM's epilogue (beta = 1) -- a conv's aggregate plus its
+        # root / skip linear, as AddLinear does for a single input block
+        Y = None if addend is None else addend.clone()
         for i, (x, w) in enumerate(zip(xs, ws)):
             last = i == n - 1
-            Y = gemm_raw(x, w, transb=True, C=Y, beta=0.0 if i == 0 else 1.0,
+            Y = gemm_raw(x, w, transb=True, C=Y, beta=0.0 if Y is None else 1.0,
                          bias=bias if i == 0 else None,
                          act=act if last else ACT_NONE, drop_p=drop_p if last else 0.0, seed=seed)
         ctx.n, ctx.act, ctx.drop_p = n, act, drop_p
@@ -673,16 +675,16 @@ class FusedLinear(torch.autograd.Function):
         gb = colsum_raw(g) if (ctx.has_bias and ctx.needs_input_grad[0]) else None
         gxs, gws = [], []
         for i in range(n):
-            gx = gemm_raw(g, ws[i]) if ctx.needs_input_grad[5 + i] else None          # dX = dY @ W
-            gw = gemm_raw(g, xs[i], transa=True) if ctx.needs_input_grad[5 + n + i] else None  # dW = dY^T @ X
+            gx = gemm_raw(g, ws[i]) if ctx.needs_input_grad[6 + i] else None          # dX = dY @ W
+            gw = gemm_raw(g, xs[i], transa=True) if ctx.needs_input_grad[6 + n + i] else None  # dW = dY^T @ X
             gxs.append(gx)
             gws.append(gw)
-        return (gb, None, None, None, None, *gxs, *gws)
+        return (gb, g if ctx.needs_input_grad[1] else None, None, None, None, None, *gxs, *gws)
 
 
-def fused_linear(xs, ws, bias=None, act=ACT_NONE, drop_p=0.0, seed=0):
+def fused_linear(xs, ws, bias=None, act=ACT_NONE, drop_p=0.0, seed=0, addend=None):
     xs, ws = list(xs), list(ws)
-    return FusedLinear.apply(bias, int(act), float(drop_p), int(seed), len(xs), *xs, *ws)
+    return FusedLinear.apply(bias, addend, int(act), float(drop_p), int(seed), len(xs), *xs, *ws)
 
 
 def aggregate_into(adj, x, out):
@@ -1054,6 +1056,88 @@ class SpMMValues(torch.autograd.Function):
         if ctx.needs_input_grad[1]:
             dv = spmm_raw(_share_plan(st.bwd, alpha[st.t_perm].contiguous()), g, use_val=True, div_rows=False)
         return dalpha, dv, None
+
+
+def attn_score_raw(plan, q, k):
+    """score[e] = <q[row(e)], k[col(e)]> for every stored entry of the CSR block behind ``plan`` (an SpMM plan over
+    the whole block, ``Structure.fwd`` / ``.bwd``), in CSR order; q [n_rows, F] and k [n_cols, F] may be column slices
+    with a leading dimension"""
+    lib = _lib.load()
+    q, k = _rowmajor(q), _rowmajor(k)
+    if getattr(plan, "subset", False):
+        raise RuntimeError("attn_score_raw needs the plan of a whole block, not a row subset")
+    if q.size(0) != plan.n_rows or k.size(0) != plan.n_cols or q.size(1) != k.size(1):
+        raise RuntimeError(f"attention score shapes: block {plan.n_rows}x{plan.n_cols}, q {tuple(q.shape)}, "
+                           f"k {tuple(k.shape)}")
+    F = q.size(1)
+    score = torch.empty(plan.nnz, dtype=torch.float32, device=q.device)
+    with profiling.span(f"attn_score_csr_f32 F={F}", plan.nnz * (F * 4 + 8) + plan.n_rows * F * 4, 2 * plan.nnz * F):
+        check(lib.plnlp_attn_score_csr_f32(ptr(plan.item_ptr), ptr(plan.item_row), plan.n_items, ptr(plan.col),
+                                           ptr(q), _ld(q), ptr(k), _ld(k), F, ptr(score), stream()),
+              "plnlp_attn_score_csr_f32")
+    return score
+
+
+def block_attention_fwd(q, k, v, st, scale):
+    """the attention of a CSR row block with separate query and key / value tables -> (score [nnz], alpha [nnz],
+    agg [n_rows, F]): per-entry scores (attn_score_raw), the per-row softmax, and the SpMM with the weights as values"""
+    from .graph import _share_plan
+    if st.fwd.nnz == 0:                       # an empty block (padding rows only): nothing to attend to
+        s = torch.empty(0, dtype=torch.float32, device=q.device)
+        return s, s, torch.zeros(st.n_rows, q.size(1), dtype=torch.float32, device=q.device)
+    s = attn_score_raw(st.fwd, q, k)
+    alpha = torch.empty_like(s)
+    lib = _lib.load()
+    with profiling.span("segment_softmax_fwd_f32", s.numel() * 8, 0):
+        check(lib.plnlp_segment_softmax_fwd_f32(ptr(st.rowptr), st.n_rows, ptr(s), float(scale), ptr(alpha), stream()),
+              "plnlp_segment_softmax_fwd_f32")
+    agg = spmm_raw(_share_plan(st.fwd, alpha), v, use_val=True, div_rows=False)
+    return s, alpha, agg
+
+
+class BlockAttention(torch.autograd.Function):
+    """agg = softmax_row(scale <q_i, k_j>) v_j over the stored entries of a row block ``adj`` [n_q, n_k] (the
+    row-partitioned TransformerConv).  q [n_q, F] holds the block's own rows; kv [n_k, 2F] = [k | v] holds every
+    gathered row.  Backward, on the plans the block's Structure already has (fixed order, deterministic):
+    dalpha = score(g, v), ds = softmax backward, dq = A(ds) k, dk = A(ds)^T q, dv = A(alpha)^T g -- dk and dv
+    written side by side into one [n_k, 2F] gradient of kv."""
+
+    @staticmethod
+    def forward(ctx, q, kv, adj, scale):
+        st = structure_of(adj)
+        F = q.size(1)
+        _, alpha, agg = block_attention_fwd(q, kv[:, :F], kv[:, F:], st, scale)
+        ctx.st, ctx.scale = st, float(scale)
+        ctx.save_for_backward(q, kv, alpha)
+        return agg
+
+    @staticmethod
+    def backward(ctx, g):
+        from .graph import _share_plan
+        q, kv, alpha = ctx.saved_tensors
+        st, F = ctx.st, q.size(1)
+        if st.fwd.nnz == 0:
+            return torch.zeros_like(q), torch.zeros_like(kv), None, None
+        g = _rowmajor(g)
+        k, v = kv[:, :F], kv[:, F:]
+        dalpha = attn_score_raw(st.fwd, g, v)
+        ds = torch.empty_like(alpha)
+        lib = _lib.load()
+        with profiling.span("segment_softmax_bwd_f32", alpha.numel() * 12, 0):
+            check(lib.plnlp_segment_softmax_bwd_f32(ptr(st.rowptr), st.n_rows, ptr(alpha), ptr(dalpha), ctx.scale,
+                                                    ptr(ds), stream()), "plnlp_segment_softmax_bwd_f32")
+        dq = spmm_raw(_share_plan(st.fwd, ds), k, use_val=True, div_rows=False) if ctx.needs_input_grad[0] else None
+        dkv = None
+        if ctx.needs_input_grad[1]:
+            dkv = torch.empty(kv.size(0), 2 * F, dtype=torch.float32, device=kv.device)
+            spmm_raw(_share_plan(st.bwd, ds[st.t_perm].contiguous()), q, use_val=True, div_rows=False, out=dkv[:, :F])
+            spmm_raw(_share_plan(st.bwd, alpha[st.t_perm].contiguous()), g, use_val=True, div_rows=False,
+                     out=dkv[:, F:])
+        return dq, dkv, None, None
+
+
+def block_attention(q, kv, adj, scale):
+    return BlockAttention.apply(q, kv, adj, float(scale))
 
 
 class AddLinear(torch.autograd.Function):

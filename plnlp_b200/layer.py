@@ -274,7 +274,12 @@ class TransformerConv(torch.nn.Module):
 
     Kernels: four tcgen05 GEMMs, the edge-dot kernel over the stored entries for the scores, a per-row softmax
     (csrc/attn.cu), the SpMM kernel with the attention weights as values, and the skip connection accumulated in
-    a GEMM epilogue.  Parameters: lin_key / lin_query / lin_value / lin_skip (.weight, .bias)."""
+    a GEMM epilogue.  Parameters: lin_key / lin_query / lin_value / lin_skip (.weight, .bias).
+
+    On a row-partitioned adjacency (``parallel.ShardedAdj``) rank r holds rows [lo, hi) of x and the row block
+    A[lo:hi, :].  Every input block is all-gathered (``parallel.gather_rows``; backward: the reduce-scatter of its
+    gradient), key and value of ALL rows come from one GEMM with the two weights stacked, queries and the skip term
+    from the local rows only, and the block's attention runs in ``forward_block`` (DESIGN.md section 6)."""
 
     def __init__(self, in_channels, out_channels, heads=1):
         super().__init__()
@@ -290,10 +295,14 @@ class TransformerConv(torch.nn.Module):
         for lin in (self.lin_key, self.lin_query, self.lin_value, self.lin_skip):
             lin.reset_parameters()
 
-    def forward(self, x, adj_t, act=_ops.ACT_NONE, drop_p=0.0, sparse_grad=False):
+    def forward(self, x, adj_t, act=_ops.ACT_NONE, drop_p=0.0, sparse_grad=False, attention=None):
+        """``attention`` (row-partitioned adjacency only): the per-block attention ``attention(q, kv, adj, scale)``,
+        by default ``_ops.block_attention``; a test can put a reference restatement in its place."""
         from . import parallel
         if isinstance(adj_t, parallel.ShardedAdj):
-            raise NotImplementedError("TransformerConv on a row-partitioned adjacency")
+            parts = _as_parts(x)
+            fulls = [_gather_input(p, adj_t) for p in parts]
+            return self.forward_block(parts, fulls, adj_t.local, act, drop_p, attention)
         parts = _as_parts(x)
         x = parts[0] if len(parts) == 1 else torch.cat(parts, -1)
         st = _ops.structure_of(adj_t)
@@ -303,6 +312,36 @@ class TransformerConv(torch.nn.Module):
         agg = _ops.SpMMValues.apply(alpha, v, adj_t)
         return _ops.AddLinear.apply(x, self.lin_skip.weight, self.lin_skip.bias, agg, int(act), float(drop_p),
                                     _ops.new_seed() if drop_p > 0 else 0)
+
+    def forward_block(self, parts, fulls, adj, act=_ops.ACT_NONE, drop_p=0.0, attention=None):
+        """the conv on one row block, no collective: ``parts`` are the block's own rows of every input block,
+        ``fulls`` the same blocks over every column of ``adj`` (the block's rows of the adjacency).  The linears run
+        on column slices of the weights, one GEMM per input block, so [emb | x] is never concatenated."""
+        q = _ops.fused_linear(parts, _split_cols(self.lin_query.weight, parts), self.lin_query.bias)
+        w_kv = torch.cat([self.lin_key.weight, self.lin_value.weight], 0)      # one GEMM -> [n_cols, 2F] = [k | v]
+        b_kv = torch.cat([self.lin_key.bias, self.lin_value.bias], 0)
+        kv = _ops.fused_linear(fulls, _split_cols(w_kv, fulls), b_kv)
+        agg = (attention or _ops.block_attention)(q, kv, adj, 1.0 / math.sqrt(self.out_channels))
+        return _ops.fused_linear(parts, _split_cols(self.lin_skip.weight, parts), self.lin_skip.bias, act, drop_p,
+                                 _ops.new_seed() if drop_p > 0 else 0, addend=agg)
+
+
+def _gather_input(x_local, sadj):
+    """all rows [R*blk, w] of a row-partitioned input block.  A block marked constant (``mark_constant``: data.x) is
+    gathered once and kept on the adjacency object, keyed on its storage, shape and version counter like
+    ``_const_aggregate``; any other block goes through ``parallel.gather_rows`` (backward: reduce-scatter)."""
+    from . import parallel
+    if not _is_const(x_local):
+        return parallel.gather_rows(parallel.pad_rows(x_local, sadj.blk), sadj.group, tag="attention input")
+    cache = sadj.__dict__.setdefault("_plnlp_const_gather", {})
+    key = (x_local.data_ptr(), tuple(x_local.shape), x_local.stride(0), x_local._version)
+    hit = cache.get(key)
+    if hit is None:
+        cache.clear()                       # one constant block per adjacency: never hold stale copies
+        with torch.no_grad():
+            hit = cache[key] = parallel.all_gather_rows(parallel.pad_rows(x_local, sadj.blk), sadj.group,
+                                                        name="nccl all_gather (constant attention input)")
+    return hit
 
 
 class BaseGNN(torch.nn.Module):
