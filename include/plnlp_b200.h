@@ -445,6 +445,16 @@ int plnlp_subset_plan_fill(const int64_t* rowptr, const int64_t* rows, int64_t T
                            int32_t* item_end, int32_t* item_row, int32_t* item_slot, int32_t* fix_ptr,
                            int32_t* fix_row, float* row_cnt, void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * Common-neighbour link heuristics (plnlp_b200/heuristics.py; csrc/heuristic.cu): CN, Adamic-Adar and Resource
+ * Allocation, the non-learned baselines of the OGB link-prediction tables.  rowptr int64 [n + 1] / col int32 [nnz]:
+ * a cleaned CSR (every row sorted, distinct, without its diagonal entry).  out[p] (fp64) = the sum over the common
+ * neighbours w of rows edges[p, 0] and edges[p, 1] of weight[w] (fp64 [n]), or their count when weight is NULL.
+ * edges int64 [P, 2] with ids in [0, n).  Run-to-run deterministic.
+ * ------------------------------------------------------------------------------------ */
+int plnlp_link_heuristic_f64(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz, const double* weight,
+                             const int64_t* edges, int64_t P, double* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1309,3 +1309,21 @@ def topk_merge_raw(ids_in, scores_in, k):
         check(lib.plnlp_topk_merge_f32(ptr(ids_in), ptr(scores_in), R, Q, k_in, int(k), ptr(ids), ptr(scores),
                                        stream()), "plnlp_topk_merge_f32")
     return ids, scores
+
+
+def link_heuristic_raw(rowptr, col, weight, edges):
+    """fp64 [P]: for every pair edges[p] = (u, v) (int64 [P, 2], ids in [0, n)) the sum of ``weight[w]`` (fp64 [n])
+    over the common neighbours w of rows u and v of the cleaned CSR (rowptr int64 [n + 1], col int32), or their count
+    when ``weight`` is None (heuristics.py)"""
+    lib = _lib.load()
+    if rowptr.dtype != torch.int64 or col.dtype != torch.int32 or edges.dtype != torch.int64:
+        raise RuntimeError("link_heuristic_raw: rowptr and edges must be int64, col int32")
+    if weight is not None and weight.dtype != torch.float64:
+        raise RuntimeError("link_heuristic_raw: weight must be fp64")
+    P = edges.size(0)
+    out = torch.empty(P, dtype=torch.float64, device=edges.device)
+    with profiling.span("link_heuristic_f64", P * 16, 0):
+        check(lib.plnlp_link_heuristic_f64(ptr(rowptr.contiguous()), ptr(col.contiguous()), rowptr.numel() - 1,
+                                           col.numel(), ptr(None if weight is None else weight.contiguous()),
+                                           ptr(edges.contiguous()), P, ptr(out), stream()), "plnlp_link_heuristic_f64")
+    return out
