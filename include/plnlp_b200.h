@@ -454,6 +454,26 @@ int plnlp_subset_plan_fill(const int64_t* rowptr, const int64_t* rows, int64_t T
  * ------------------------------------------------------------------------------------ */
 int plnlp_link_heuristic_f64(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz, const double* weight,
                              const int64_t* edges, int64_t P, double* out, void* stream);
+/* Heuristic recommendation over all nodes (plnlp_b200/heuristics.py recommend / rank_against_all): a chunk of Qc
+ * query nodes against W candidate columns, the nodes [col0, col0 + W) or, with cand != NULL (strictly ascending
+ * global ids, col0 must then be 0, else PLNLP_E_UNSUPPORTED), the nodes cand[0 .. W).
+ * Mark: bitmap uint32 [Qc, ceil(W / 32)], zeroed by the caller; bit c of row q is set when column c's node j lies
+ * in R(w) = {j : w in N(j)} for some w in N(nodes[q]) -- the nodes sharing a neighbour with the query.  rowptr / col:
+ * the cleaned table N; rrowptr / rcol: its transpose R (same n); item_ptr int64 [Qc + 1]: item_ptr[0] = 0 and
+ * item_ptr[q + 1] - item_ptr[q] = |N(nodes[q])|.  Every pointer but cand is required when Qc > 0 and W > 0 (a table
+ * without entries marks nothing: skip the call).  The final bitmap does not depend on the order of the writes. */
+int plnlp_two_hop_mark(const int64_t* rowptr, const int32_t* col, const int64_t* rrowptr, const int32_t* rcol,
+                       int64_t n, const int64_t* nodes, const int64_t* item_ptr, int64_t Qc, int64_t col0, int64_t W,
+                       const int64_t* cand, uint32_t* bitmap, void* stream);
+/* Score: s [Qc, W] (row stride lds >= W), zeroed by the caller.  For every set bit c of row q, s[q, c] = the value
+ * plnlp_link_heuristic_f64 gives the pair (nodes[q], column c's node) -- the same routine, bit for bit -- rounded to
+ * fp32 once (_f32) or kept in fp64 (_f64).  Unmarked entries are not written. */
+int plnlp_two_hop_score_f32(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz, const double* weight,
+                            const int64_t* nodes, int64_t Qc, int64_t col0, int64_t W, const int64_t* cand,
+                            const uint32_t* bitmap, float* s, int64_t lds, void* stream);
+int plnlp_two_hop_score_f64(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz, const double* weight,
+                            const int64_t* nodes, int64_t Qc, int64_t col0, int64_t W, const int64_t* cand,
+                            const uint32_t* bitmap, double* s, int64_t lds, void* stream);
 
 #ifdef __cplusplus
 }

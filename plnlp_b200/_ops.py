@@ -1327,3 +1327,54 @@ def link_heuristic_raw(rowptr, col, weight, edges):
                                            col.numel(), ptr(None if weight is None else weight.contiguous()),
                                            ptr(edges.contiguous()), P, ptr(out), stream()), "plnlp_link_heuristic_f64")
     return out
+
+
+def _two_hop_args(rowptr, col, nodes, W, col0, cand):
+    if rowptr.dtype != torch.int64 or col.dtype != torch.int32 or nodes.dtype != torch.int64:
+        raise RuntimeError("two_hop: rowptr and nodes must be int64, col int32")
+    if cand is not None:
+        cand = _cand_ids(cand, W)
+        if col0 != 0:
+            raise RuntimeError("two_hop: a candidate chunk has col0 = 0")
+    return rowptr.contiguous(), col.contiguous(), nodes.contiguous(), cand
+
+
+def two_hop_mark_raw(rowptr, col, rrowptr, rcol, nodes, W, col0=0, cand=None):
+    """int32 [Qc, ceil(W / 32)] bitmap (read as uint32): bit c of row q is set when column c's node -- col0 + c, or
+    cand[c] -- shares a neighbour with nodes[q]: it lies in row w of the transposed table (rrowptr int64, rcol int32)
+    for some w in row nodes[q] of the cleaned table (rowptr int64, col int32) (heuristics.py)"""
+    lib = _lib.load()
+    rowptr, col, nodes, cand = _two_hop_args(rowptr, col, nodes, W, col0, cand)
+    if rrowptr.dtype != torch.int64 or rcol.dtype != torch.int32 or rrowptr.numel() != rowptr.numel():
+        raise RuntimeError("two_hop_mark_raw: the transposed table is int64 rrowptr + int32 rcol over the same nodes")
+    Qc = nodes.numel()
+    bitmap = torch.zeros(Qc, (W + 31) // 32, dtype=torch.int32, device=nodes.device)
+    if col.numel() == 0 or rcol.numel() == 0:         # a table without entries (an empty block) reaches nothing
+        return bitmap
+    item_ptr = torch.zeros(Qc + 1, dtype=torch.int64, device=nodes.device)
+    item_ptr[1:] = torch.cumsum(rowptr[nodes + 1] - rowptr[nodes], 0)
+    with profiling.span("two_hop_mark", 0, 0):
+        check(lib.plnlp_two_hop_mark(ptr(rowptr), ptr(col), ptr(rrowptr.contiguous()), ptr(rcol.contiguous()),
+                                     rowptr.numel() - 1, ptr(nodes), ptr(item_ptr), Qc, int(col0), int(W), ptr(cand),
+                                     ptr(bitmap), stream()), "plnlp_two_hop_mark")
+    return bitmap
+
+
+def two_hop_score_raw(rowptr, col, weight, nodes, bitmap, W, col0=0, cand=None, dtype=torch.float32):
+    """S [Qc, W] in ``dtype`` (fp32: each sum rounded once; fp64: kept): for every set bit of ``bitmap``
+    (``two_hop_mark_raw``) the ``link_heuristic_raw`` value of the pair (nodes[q], column c's node), bit for bit; 0
+    elsewhere"""
+    lib = _lib.load()
+    rowptr, col, nodes, cand = _two_hop_args(rowptr, col, nodes, W, col0, cand)
+    if weight is not None and weight.dtype != torch.float64:
+        raise RuntimeError("two_hop_score_raw: weight must be fp64")
+    Qc = nodes.numel()
+    if bitmap.dtype != torch.int32 or tuple(bitmap.shape) != (Qc, (W + 31) // 32):
+        raise RuntimeError("two_hop_score_raw: bitmap must be the int32 [Qc, ceil(W / 32)] of two_hop_mark_raw")
+    s = torch.zeros(Qc, W, dtype=dtype, device=nodes.device)
+    f = {torch.float32: lib.plnlp_two_hop_score_f32, torch.float64: lib.plnlp_two_hop_score_f64}[dtype]
+    with profiling.span(f"two_hop_score_{'f32' if dtype == torch.float32 else 'f64'}", 0, 0):
+        check(f(ptr(rowptr), ptr(col), rowptr.numel() - 1, col.numel(),
+                ptr(None if weight is None else weight.contiguous()), ptr(nodes), Qc, int(col0), int(W), ptr(cand),
+                ptr(bitmap.contiguous()), ptr(s), W, stream()), "plnlp_two_hop_score")
+    return s

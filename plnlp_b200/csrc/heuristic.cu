@@ -26,6 +26,67 @@ __device__ __forceinline__ int ilog2_ceil(int64_t x) {
     return 64 - __clzll(static_cast<unsigned long long>(x));
 }
 
+// the sum of weight[w] (1 when weight == NULL) over w in N(u) & N(v), computed by the whole warp and returned to
+// every lane: the cheaper of the two intersections above, lane terms in list order, then the fixed butterfly.  The
+// argument order matters only for equal lengths (u's list is then the "shorter" one); callers pass (query, other).
+__device__ __forceinline__ double warp_common_neighbours(const int64_t* __restrict__ rowptr,
+                                                         const int32_t* __restrict__ col,
+                                                         const double* __restrict__ weight, int64_t u, int64_t v,
+                                                         int lane) {
+    int64_t a0 = __ldg(rowptr + u), a1 = __ldg(rowptr + u + 1);
+    int64_t b0 = __ldg(rowptr + v), b1 = __ldg(rowptr + v + 1);
+    if (a1 - a0 > b1 - b0) {                    // a: the shorter list
+        int64_t t = a0; a0 = b0; b0 = t;
+        t = a1; a1 = b1; b1 = t;
+    }
+    const int64_t la = a1 - a0, lb = b1 - b0;
+    const int32_t* A = col + a0;
+    const int32_t* B = col + b0;
+    double acc = 0.0;
+    if (la > 0) {
+        const int64_t steps_search = ((la + 31) >> 5) * ilog2_ceil(lb);
+        const int64_t steps_merge = ((la + lb + 31) >> 5) + ilog2_ceil(la);
+        if (steps_search <= steps_merge) {
+            int64_t lo = 0;
+            for (int64_t i = lane; i < la; i += 32) {
+                const int32_t w = __ldg(A + i);
+                int64_t hi = lb;
+                while (lo < hi) {                   // lower bound of w in B[lo, lb)
+                    const int64_t m = (lo + hi) >> 1;
+                    if (__ldg(B + m) < w) lo = m + 1; else hi = m;
+                }
+                if (lo < lb && __ldg(B + lo) == w) acc += weight ? __ldg(weight + w) : 1.0;
+            }
+        } else {
+            const int64_t L = la + lb;
+            const int64_t d0 = (L * lane) >> 5, d1 = (L * (lane + 1)) >> 5;
+            // i = entries of A among the first d0 of the merge (A first on ties): the largest i with
+            // A[i - 1] <= B[d0 - i]
+            int64_t lo = d0 > lb ? d0 - lb : 0, hi = d0 < la ? d0 : la;
+            while (lo < hi) {
+                const int64_t m = (lo + hi) >> 1;
+                if (__ldg(A + m) <= __ldg(B + d0 - m - 1)) lo = m + 1; else hi = m;
+            }
+            int64_t i = lo, j = d0 - lo;
+            int32_t x = i < la ? __ldg(A + i) : INT32_MAX;
+            int32_t y = j < lb ? __ldg(B + j) : INT32_MAX;
+            for (int64_t d = d0; d < d1; ++d) {
+                if (i < la && (j >= lb || x <= y)) {
+                    if (x == y) acc += weight ? __ldg(weight + x) : 1.0;
+                    ++i;
+                    x = i < la ? __ldg(A + i) : INT32_MAX;
+                } else {
+                    ++j;
+                    y = j < lb ? __ldg(B + j) : INT32_MAX;
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    return acc;
+}
+
 __global__ void __launch_bounds__(kHeurThreads) link_heuristic_kernel(const int64_t* __restrict__ rowptr,
                                                                      const int32_t* __restrict__ col,
                                                                      const double* __restrict__ weight,
@@ -35,59 +96,101 @@ __global__ void __launch_bounds__(kHeurThreads) link_heuristic_kernel(const int6
     const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
     for (int64_t p = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; p < P; p += n_warps) {
         const int64_t u = __ldg(edges + 2 * p), v = __ldg(edges + 2 * p + 1);
-        int64_t a0 = __ldg(rowptr + u), a1 = __ldg(rowptr + u + 1);
-        int64_t b0 = __ldg(rowptr + v), b1 = __ldg(rowptr + v + 1);
-        if (a1 - a0 > b1 - b0) {                    // a: the shorter list
-            int64_t t = a0; a0 = b0; b0 = t;
-            t = a1; a1 = b1; b1 = t;
-        }
-        const int64_t la = a1 - a0, lb = b1 - b0;
-        const int32_t* A = col + a0;
-        const int32_t* B = col + b0;
-        double acc = 0.0;
-        if (la > 0) {
-            const int64_t steps_search = ((la + 31) >> 5) * ilog2_ceil(lb);
-            const int64_t steps_merge = ((la + lb + 31) >> 5) + ilog2_ceil(la);
-            if (steps_search <= steps_merge) {
-                int64_t lo = 0;
-                for (int64_t i = lane; i < la; i += 32) {
-                    const int32_t w = __ldg(A + i);
-                    int64_t hi = lb;
-                    while (lo < hi) {                   // lower bound of w in B[lo, lb)
-                        const int64_t m = (lo + hi) >> 1;
-                        if (__ldg(B + m) < w) lo = m + 1; else hi = m;
-                    }
-                    if (lo < lb && __ldg(B + lo) == w) acc += weight ? __ldg(weight + w) : 1.0;
-                }
-            } else {
-                const int64_t L = la + lb;
-                const int64_t d0 = (L * lane) >> 5, d1 = (L * (lane + 1)) >> 5;
-                // i = entries of A among the first d0 of the merge (A first on ties): the largest i with
-                // A[i - 1] <= B[d0 - i]
-                int64_t lo = d0 > lb ? d0 - lb : 0, hi = d0 < la ? d0 : la;
-                while (lo < hi) {
-                    const int64_t m = (lo + hi) >> 1;
-                    if (__ldg(A + m) <= __ldg(B + d0 - m - 1)) lo = m + 1; else hi = m;
-                }
-                int64_t i = lo, j = d0 - lo;
-                int32_t x = i < la ? __ldg(A + i) : INT32_MAX;
-                int32_t y = j < lb ? __ldg(B + j) : INT32_MAX;
-                for (int64_t d = d0; d < d1; ++d) {
-                    if (i < la && (j >= lb || x <= y)) {
-                        if (x == y) acc += weight ? __ldg(weight + x) : 1.0;
-                        ++i;
-                        x = i < la ? __ldg(A + i) : INT32_MAX;
-                    } else {
-                        ++j;
-                        y = j < lb ? __ldg(B + j) : INT32_MAX;
-                    }
-                }
-            }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+        const double acc = warp_common_neighbours(rowptr, col, weight, u, v, lane);
         if (lane == 0) out[p] = acc;
     }
+}
+
+// the column of node j in a chunk: j - col0 when it lies in [col0, col0 + W), or, with cand (strictly ascending,
+// W entries), its position there; -1 when the chunk has no such column
+__device__ __forceinline__ int64_t chunk_column(const int64_t* __restrict__ cand, int64_t col0, int64_t W, int64_t j) {
+    if (cand == nullptr) return j >= col0 && j - col0 < W ? j - col0 : -1;
+    int64_t lo = 0, hi = W;
+    while (lo < hi) {
+        const int64_t m = (lo + hi) >> 1;
+        if (__ldg(cand + m) < j) lo = m + 1; else hi = m;
+    }
+    return lo < W && __ldg(cand + lo) == j ? lo : -1;
+}
+
+// Mark: work item t in [0, item_ptr[Qc]) is (query qi, the (t - item_ptr[qi])-th w of N(nodes[qi])); one warp per
+// item, items strided over the warps of the grid, lanes strided over R(w).  Every j of R(w) that has a column sets
+// its bit; atomicOr makes the bitmap independent of the order.
+__global__ void __launch_bounds__(kHeurThreads) two_hop_mark_kernel(
+    const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int64_t* __restrict__ rrowptr,
+    const int32_t* __restrict__ rcol, const int64_t* __restrict__ nodes, const int64_t* __restrict__ item_ptr,
+    int64_t Qc, int64_t col0, int64_t W, const int64_t* __restrict__ cand, uint32_t* __restrict__ bitmap,
+    int64_t words) {
+    const int lane = threadIdx.x & 31;
+    const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+    const int64_t total = __ldg(item_ptr + Qc);
+    for (int64_t t = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; t < total; t += n_warps) {
+        int64_t lo = 0, hi = Qc;                    // the query: the last qi with item_ptr[qi] <= t
+        while (hi - lo > 1) {
+            const int64_t m = (lo + hi) >> 1;
+            if (__ldg(item_ptr + m) <= t) lo = m; else hi = m;
+        }
+        const int64_t w = __ldg(col + __ldg(rowptr + __ldg(nodes + lo)) + (t - __ldg(item_ptr + lo)));
+        uint32_t* row = bitmap + lo * words;
+        const int64_t r1 = __ldg(rrowptr + w + 1);
+        for (int64_t e = __ldg(rrowptr + w) + lane; e < r1; e += 32) {
+            const int64_t c = chunk_column(cand, col0, W, __ldg(rcol + e));
+            if (c >= 0) atomicOr(row + (c >> 5), 1u << (c & 31));
+        }
+    }
+}
+
+// Score: the bitmap [Qc, words] flattened; a warp takes runs of 32 words (one per lane, one coalesced load), skips
+// the empty ones by ballot and, for every set bit of the others, intersects N(nodes[q]) with N(j) through
+// warp_common_neighbours -- the routine of link_heuristic_kernel, so each entry equals that kernel's result for the
+// pair (nodes[q], j) bit for bit.  Unmarked entries are left as they are (the caller zeroes s).
+template <class T>
+__global__ void __launch_bounds__(kHeurThreads) two_hop_score_kernel(
+    const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col, const double* __restrict__ weight,
+    const int64_t* __restrict__ nodes, int64_t Qc, int64_t col0, const int64_t* __restrict__ cand,
+    const uint32_t* __restrict__ bitmap, int64_t words, T* __restrict__ s, int64_t lds) {
+    const int lane = threadIdx.x & 31;
+    const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+    const int64_t total = Qc * words;
+    for (int64_t g0 = ((static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5) * 32; g0 < total;
+         g0 += n_warps * 32) {
+        const int64_t g = g0 + lane;
+        const uint32_t mine = g < total ? __ldg(bitmap + g) : 0u;
+        unsigned live = __ballot_sync(0xffffffffu, mine != 0u);
+        while (live) {
+            const int src = __ffs(live) - 1;
+            live &= live - 1;
+            uint32_t bits = __shfl_sync(0xffffffffu, mine, src);
+            const int64_t gw = g0 + src;
+            const int64_t q = gw / words;
+            const int64_t c_base = (gw - q * words) * 32;
+            const int64_t u = __ldg(nodes + q);
+            while (bits) {
+                const int b = __ffs(static_cast<int>(bits)) - 1;
+                bits &= bits - 1;
+                const int64_t c = c_base + b;
+                const int64_t j = cand != nullptr ? __ldg(cand + c) : col0 + c;
+                const double acc = warp_common_neighbours(rowptr, col, weight, u, j, lane);
+                if (lane == 0) s[q * lds + c] = static_cast<T>(acc);
+            }
+        }
+    }
+}
+
+template <class T>
+int two_hop_score(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz, const double* weight,
+                  const int64_t* nodes, int64_t Qc, int64_t col0, int64_t W, const int64_t* cand,
+                  const uint32_t* bitmap, T* s, int64_t lds, void* stream) {
+    PLNLP_REQUIRE(n >= 0 && nnz >= 0 && Qc >= 0 && W >= 0 && col0 >= 0 && lds >= W, PLNLP_E_SIZE);
+    if (Qc == 0 || W == 0) return 0;
+    PLNLP_REQUIRE(n > 0, PLNLP_E_SIZE);
+    PLNLP_REQUIRE(rowptr && nodes && bitmap && s && (nnz == 0 || col), PLNLP_E_NULL);
+    const int64_t words = ceil_div(W, 32);
+    const int64_t blocks = std::min<int64_t>(ceil_div(Qc * words, kHeurThreads), int64_t(kNumSM) * 8);
+    two_hop_score_kernel<T><<<static_cast<unsigned>(blocks), kHeurThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        rowptr, col, weight, nodes, Qc, col0, cand, bitmap, words, s, lds);
+    PLNLP_LAUNCH_CHECK();
+    return 0;
 }
 
 }  // namespace
@@ -107,4 +210,46 @@ extern "C" int plnlp_link_heuristic_f64(const int64_t* rowptr, const int32_t* co
                                    static_cast<cudaStream_t>(stream)>>>(rowptr, col, weight, edges, P, out);
     PLNLP_LAUNCH_CHECK();
     return 0;
+}
+
+// bitmap uint32 [Qc, ceil(W / 32)], zeroed by the caller: bit c of row qi is set when column c's node j is reachable
+// from nodes[qi] in two steps, j in R(w) for some w in N(nodes[qi]).  rowptr / col: the cleaned table N; rrowptr /
+// rcol: its transpose R; item_ptr int64 [Qc + 1]: the running sum of |N(nodes[qi])|, item_ptr[0] = 0.  Columns: the
+// nodes [col0, col0 + W), or cand[0 .. W) (strictly ascending) when cand != NULL (then col0 = 0).
+extern "C" int plnlp_two_hop_mark(const int64_t* rowptr, const int32_t* col, const int64_t* rrowptr,
+                                  const int32_t* rcol, int64_t n, const int64_t* nodes, const int64_t* item_ptr,
+                                  int64_t Qc, int64_t col0, int64_t W, const int64_t* cand, uint32_t* bitmap,
+                                  void* stream) {
+    PLNLP_REQUIRE(n >= 0 && Qc >= 0 && W >= 0 && col0 >= 0, PLNLP_E_SIZE);
+    PLNLP_REQUIRE(cand == nullptr || col0 == 0, PLNLP_E_UNSUPPORTED);
+    if (Qc == 0 || W == 0) return 0;
+    PLNLP_REQUIRE(n > 0, PLNLP_E_SIZE);
+    PLNLP_REQUIRE(rowptr && col && rrowptr && rcol && nodes && item_ptr && bitmap, PLNLP_E_NULL);
+    const int64_t words = plnlp::ceil_div(W, 32);
+    const int64_t blocks = int64_t(plnlp::kNumSM) * 8;      // the item count stays on the device
+    plnlp::two_hop_mark_kernel<<<static_cast<unsigned>(blocks), plnlp::kHeurThreads, 0,
+                                 static_cast<cudaStream_t>(stream)>>>(rowptr, col, rrowptr, rcol, nodes, item_ptr, Qc,
+                                                                      col0, W, cand, bitmap, words);
+    PLNLP_LAUNCH_CHECK();
+    return 0;
+}
+
+// s [Qc, W] (row stride lds), zeroed by the caller: for every set bit c of row qi of the bitmap of
+// plnlp_two_hop_mark, s[qi, c] = the sum of plnlp_link_heuristic_f64 for the pair (nodes[qi], column c's node),
+// rounded to fp32 once (_f32) or kept in fp64 (_f64).  Same table, weight and column forms as above.
+extern "C" int plnlp_two_hop_score_f32(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz,
+                                       const double* weight, const int64_t* nodes, int64_t Qc, int64_t col0,
+                                       int64_t W, const int64_t* cand, const uint32_t* bitmap, float* s, int64_t lds,
+                                       void* stream) {
+    PLNLP_REQUIRE(cand == nullptr || col0 == 0, PLNLP_E_UNSUPPORTED);
+    return plnlp::two_hop_score<float>(rowptr, col, n, nnz, weight, nodes, Qc, col0, W, cand, bitmap, s, lds, stream);
+}
+
+extern "C" int plnlp_two_hop_score_f64(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz,
+                                       const double* weight, const int64_t* nodes, int64_t Qc, int64_t col0,
+                                       int64_t W, const int64_t* cand, const uint32_t* bitmap, double* s,
+                                       int64_t lds, void* stream) {
+    PLNLP_REQUIRE(cand == nullptr || col0 == 0, PLNLP_E_UNSUPPORTED);
+    return plnlp::two_hop_score<double>(rowptr, col, n, nnz, weight, nodes, Qc, col0, W, cand, bitmap, s, lds,
+                                        stream);
 }

@@ -25,12 +25,28 @@ A[:, lo:hi], the transpose of the rank's row block of A^T (``ShardedAdj.local_t`
 a CSR with one row per node of the graph.  The weights of the rank's own w come from its own rows of A
 (``ShardedAdj.local``), so no degree crosses the interconnect.  The same kernel produces the fp64 partials, one fp64
 all-reduce sums them and the result is rounded to fp32 once.  ``Shard`` is the per-rank step, with no collective.
+
+``recommend`` and ``rank_against_all`` rank every node (or a candidate set) for a query, with the interface, tie rule
+and filtering of the model's calls in recommend.py.  A node outside the two-hop set of the query shares no neighbour
+with it and scores exactly +0.0, so only that set is scored: a chunk of queries against W columns is a zeroed fp32
+matrix S [Qc, W]; the mark kernel sets a bit for every j in R(w) for w in N(u) (R the transposed table, cached with
+the table), and the score kernel intersects N(u) and N(j) for every set bit with the device routine of
+``score_edges``.  Every entry therefore equals ``score_edges`` of its pair bit for bit, for every ``batch_size`` and
+on every run.  The mask and select kernels of recommend.py then run unchanged.
+
+On a row-partitioned graph both calls are collective and split the work by intermediate node as ``score_edges``
+does: rank r computes the fp64 partial of every column over w in [lo, hi), sends column block s to rank s
+(``all_to_all_single``), adds the R partials it receives in rank order 0..R-1 in fp64 and rounds once; the model's
+sharded mask, select and merge follow.  CN is exact and R = 1 is bit-identical to one GPU; AA and RA lie within one
+fp32 ulp of one GPU (and, at R >= 3, may differ by an ulp from the partitioned ``score_edges``, whose all-reduce
+sums in another order).  ``RankShard`` is the per-rank step, with no collective.
 """
 from __future__ import annotations
 
 import torch
 
-from . import _ops, graph, parallel, recommend
+from . import _ops, graph, parallel, profiling
+from . import recommend as rec
 from .utils import evaluate_hits, evaluate_mrr, get_pos_neg_edges
 
 METHODS = ("CN", "AA", "RA")
@@ -59,18 +75,30 @@ def weight_table(deg, method):
 
 class NeighbourTable:
     """the cleaned CSR the kernel intersects (``rowptr`` int64 [n + 1], ``col`` int32) and the degree d(w) of every
-    node whose weight it may read (``deg`` int64 [n]); the weight tables are built on first use"""
+    node whose weight it may read (``deg`` int64 [n]); the weight tables and the transpose are built on first use.
+    ``clean``: the cleaning function for the transpose (default ``clean_csr``)."""
 
-    def __init__(self, rowptr, col, deg=None):
+    def __init__(self, rowptr, col, deg=None, clean=None):
         self.rowptr, self.col = rowptr, col
         self.n = rowptr.numel() - 1
         self.deg = rowptr[1:] - rowptr[:-1] if deg is None else deg
         self._weights = {}
+        self._clean = clean
+        self._reach = None
 
     def weight(self, method):
         if method not in self._weights:
             self._weights[method] = weight_table(self.deg, method)
         return self._weights[method]
+
+    def reach(self):
+        """(rowptr int64 [n + 1], col int32) of the transpose R(w) = {j : w in N(j)}: ``clean_csr`` of the swapped
+        pairs.  Equal to the table itself on a symmetric graph; on any graph, j shares a neighbour with u exactly
+        when j lies in R(w) for some w in N(u)."""
+        if self._reach is None:
+            i, e = _rows_of(self.rowptr, self.n)
+            self._reach = (self._clean or clean_csr)(self.col[:e].to(torch.int64), i, self.n)
+        return self._reach
 
 
 def _rows_of(rowptr, nb):
@@ -92,7 +120,7 @@ def shard_table(local, local_t, lo, hi, n, clean=None):
     l_rowptr, l_col, _ = local.csr()
     i, e = _rows_of(l_rowptr, nb)
     own_ptr, _ = clean(lo + i, l_col[:e].to(torch.int64), n)
-    return NeighbourTable(rowptr, col, own_ptr[1:] - own_ptr[:-1])
+    return NeighbourTable(rowptr, col, own_ptr[1:] - own_ptr[:-1], clean)
 
 
 _CACHE = {}
@@ -148,13 +176,13 @@ def _score_sharded(sadj, edges, method, batch_size):
     dev = sadj.local.csr()[1].device
     e = torch.as_tensor(edges)
     try:
-        recommend._agree(sadj.group, dev, [4, e.numel(), METHODS.index(method) if method in METHODS else -1,
+        rec._agree(sadj.group, dev, [4, e.numel(), METHODS.index(method) if method in METHODS else -1,
                                            int(batch_size or 0)])
     except ValueError as err:
         raise ValueError("heuristics.score_edges on a row-partitioned graph is collective: every rank must pass "
                          "the same number of edges, method and batch_size") from err
     _check_method(method)
-    e = recommend._edge_ids(e, sadj.n_global).to(dev)
+    e = rec._edge_ids(e, sadj.n_global).to(dev)
     shard = Shard(neighbour_table(sadj))
     out = torch.empty(e.size(0), dtype=torch.float32, device=dev)
     starts, bs = _batches(e.size(0), batch_size)
@@ -174,7 +202,7 @@ def score_edges(adj_t, edges, method, batch_size=None):
     if isinstance(adj_t, parallel.ShardedAdj):
         return _score_sharded(adj_t, edges, method, batch_size)
     _check_method(method)
-    e = recommend._edge_ids(edges, adj_t.size(0))
+    e = rec._edge_ids(edges, adj_t.size(0))
     table = neighbour_table(adj_t)
     e = e.to(table.rowptr.device)
     out = torch.empty(e.size(0), dtype=torch.float32, device=e.device)
@@ -198,3 +226,325 @@ def test(data, split_edge, method, batch_size, evaluator, eval_metric):
     if eval_metric == 'hits':
         return evaluate_hits(evaluator, *preds)
     return evaluate_mrr(evaluator, *preds)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Recommendation and full ranking by a heuristic
+# ---------------------------------------------------------------------------------------------------------------------
+
+def query_bytes(W):
+    """device bytes one query row of a one-GPU chunk costs: the fp32 score row and its bitmap"""
+    return 4 * W + W // 8
+
+
+def sharded_query_bytes(W, width, R):
+    """the same for one rank of a row-partitioned graph: the fp64 partial row over all W columns, its bitmap, the
+    padded send and receive rows [R, width] (fp64) and the fp32 block row"""
+    return 8 * W + W // 8 + 16 * R * width + 4 * width
+
+
+def _chunk_rows(batch_size, row_bytes):
+    bs = int(batch_size) if batch_size else max(1, rec.CHUNK_BYTES // max(row_bytes, 1))
+    if bs < 1:
+        raise ValueError("batch_size must be positive")
+    return bs
+
+
+class Ranker:
+    """score chunks of query nodes against W columns -- the nodes [col0, col0 + W), or the candidate set ``cand``
+    (strictly ascending) -- with the table ``table``: mark the two-hop set of every query, then intersect only there.
+    ``dtype`` fp32 gives the rounded scores, fp64 a shard's partial sums.  Runs no collective."""
+
+    def __init__(self, table, method, W, col0=0, cand=None, dtype=torch.float32):
+        self.table, self.method, self.W, self.col0, self.cand, self.dtype = table, method, W, col0, cand, dtype
+
+    def chunk(self, q):
+        """S [len(q), W] in ``dtype``: the heuristic of (q[a], column c's node); exactly 0 outside the two-hop set"""
+        t = self.table
+        rrowptr, rcol = t.reach()
+        with profiling.span("heuristics: mark"):
+            bitmap = _ops.two_hop_mark_raw(t.rowptr, t.col, rrowptr, rcol, q, self.W, self.col0, self.cand)
+        with profiling.span("heuristics: score"):
+            return _ops.two_hop_score_raw(t.rowptr, t.col, t.weight(self.method), q, bitmap, self.W, self.col0,
+                                          self.cand, self.dtype)
+
+    def target_values(self, S, q, tgt):
+        """[len(q)] in S's dtype: the entry of the unmasked chunk S for (q[a], tgt[a]), or, for a target that is not
+        a column (outside ``cand``), the same value from ``link_heuristic_raw`` -- the same device routine"""
+        if self.cand is None:
+            return S.gather(1, (tgt - self.col0).reshape(-1, 1)).reshape(-1)
+        pos = torch.searchsorted(self.cand, tgt).clamp_max(max(self.W - 1, 0))
+        if self.W:
+            ts = S.gather(1, pos.reshape(-1, 1)).reshape(-1)
+            hit = self.cand[pos] == tgt
+        else:
+            ts = torch.zeros(q.numel(), dtype=self.dtype, device=q.device)
+            hit = torch.zeros(q.numel(), dtype=torch.bool, device=q.device)
+        miss = torch.nonzero(~hit).reshape(-1)
+        if miss.numel():
+            t = self.table
+            pairs = torch.stack([q[miss], tgt[miss]], 1)
+            ts[miss] = _ops.link_heuristic_raw(t.rowptr, t.col, t.weight(self.method), pairs).to(self.dtype)
+        return ts
+
+
+def _mask(S, q, rowptr, col, exclude_self, col0=0, cand=None):
+    with profiling.span("heuristics: mask"):
+        if cand is not None:
+            return _ops.score_mask_raw(S, q, rowptr, col, exclude_self, cand=cand)
+        return _ops.score_mask_raw(S, q, rowptr, col, exclude_self, col0=col0)
+
+
+def _select(S, k, t=None, ts=None, col0=0, cand=None):
+    with profiling.span("heuristics: select"):
+        if cand is not None:
+            return _ops.topk_rows_raw(S, k, target=t, target_score=ts, cand=cand)
+        return _ops.topk_rows_raw(S, k, target=t, target_score=ts, col0=col0)
+
+
+def _n_nodes(adj_t):
+    if adj_t.size(0) != adj_t.size(1):
+        raise ValueError(f"link heuristics need a square adjacency, got {adj_t.size(0)} x {adj_t.size(1)}")
+    return adj_t.size(0)
+
+
+def _exclude_edges(exclude, n, device):
+    """``exclude`` checked: None, 'adj' or an int64 [E, 2] edge tensor on the device"""
+    if exclude is None or isinstance(exclude, str):
+        if exclude is not None and exclude != "adj":
+            raise ValueError(f"exclude: expected None, 'adj' or an int64 [E, 2] edge tensor, got {exclude!r}")
+        return exclude
+    e = rec._node_ids(exclude, n, "exclude").to(device)
+    if e.dim() != 2 or e.size(1) != 2:
+        raise ValueError("exclude edges must have shape [E, 2]")
+    return e
+
+
+class RankShard:
+    """the per-rank step of the collective ``recommend`` / ``rank_against_all`` on a row-partitioned graph: rank
+    ``rank`` of ``R`` owns the intermediate nodes and the columns [lo, hi) (blocks of ``blk``), ``table`` is its
+    ``shard_table``, ``rowptr`` / ``col`` its known links (``recommend.shard_exclude_csr``).  ``cand``: the whole
+    candidate set (sorted); the rank then owns its slice of it.  Runs no collective: ``partial`` gives the fp64
+    partial of every column, laid out per owner for ``all_to_all_single``; ``combine`` adds what the rank receives
+    in rank order; ``topk`` / ``counts`` are the model's sharded tail on the rank's block."""
+
+    def __init__(self, table, method, n, rank, R, rowptr=None, col=None, exclude_self=True, cand=None):
+        from . import parallel
+        self.n, self.rank, self.R = n, rank, R
+        self.blk = parallel.block_size(n, R)
+        self.lo, self.hi = parallel.row_block(n, rank, R)
+        self.rowptr, self.col, self.exclude_self = rowptr, col, exclude_self
+        self.cand = cand
+        if cand is None:
+            self.mine, self.width, self.own = None, self.blk, self.hi - self.lo
+            self.ranker = Ranker(table, method, R * self.blk, dtype=torch.float64)
+        else:
+            self.slices = rec.candidate_slices(cand, [parallel.row_block(n, r, R) for r in range(R)])
+            a, b = self.slices[rank]
+            self.mine, self.own = cand[a:b], b - a
+            self.width = max(y - x for x, y in self.slices)
+            self.ranker = Ranker(table, method, cand.numel(), cand=cand, dtype=torch.float64)
+
+    def batch_size(self, batch_size):
+        return _chunk_rows(batch_size, sharded_query_bytes(self.ranker.W, self.width, self.R))
+
+    def partial(self, q):
+        """(P fp64 [Qc, W], send fp64 [R, Qc, width]): the rank's partial sums over its intermediate nodes for every
+        column, and the same laid out as one padded column block per owner"""
+        P = self.ranker.chunk(q)
+        Qc = q.numel()
+        if self.cand is None:
+            return P, P.view(Qc, self.R, self.blk).transpose(0, 1).contiguous()
+        send = torch.zeros(self.R, Qc, self.width, dtype=torch.float64, device=q.device)
+        for r, (a, b) in enumerate(self.slices):
+            send[r, :, :b - a] = P[:, a:b]
+        return P, send
+
+    def combine(self, recv):
+        """fp32 [Qc, own]: the R partials of the rank's columns (recv [R, Qc, width], from ranks 0 .. R-1) added in
+        rank order in fp64 and rounded once"""
+        acc = recv[0].clone()
+        for r in range(1, self.R):
+            acc += recv[r]
+        return acc[:, :self.own].to(torch.float32).contiguous()
+
+    @staticmethod
+    def target_scores(parts):
+        """fp32 [Qc] from the all-gathered target partials [R, Qc], added in rank order like ``combine``"""
+        acc = parts[0].clone()
+        for r in range(1, parts.size(0)):
+            acc += parts[r]
+        return acc.to(torch.float32)
+
+    def topk(self, S, q, k):
+        """-> (ids int64 [Qc, k] global, scores [Qc, k]): the best k of the rank's block"""
+        if self.own == 0:
+            return rec._no_candidates(q.numel(), k, q.device)
+        _mask(S, q, self.rowptr, self.col, self.exclude_self, self.lo, self.mine)
+        ids, sc, _, _ = _select(S, k, col0=self.lo, cand=self.mine)
+        return ids, sc
+
+    def counts(self, S, q, t, ts):
+        """-> int32 [2, Qc]: the rank's gt / ge counts against the target scores"""
+        if self.own == 0:
+            return torch.zeros(2, q.numel(), dtype=torch.int32, device=q.device)
+        _mask(S, q, self.rowptr, self.col, self.exclude_self, self.lo, self.mine)
+        _, _, gt, ge = _select(S, 0, t, ts, col0=self.lo, cand=self.mine)
+        return torch.stack([gt, ge])
+
+
+def _sharded_setup(sadj, call, n_items, k, method, exclude, exclude_self, batch_size, candidates):
+    """the argument check every rank runs before any other collective -> (device, candidate set or None)"""
+    dev = sadj.local.csr()[1].device
+    try:
+        rec._agree(sadj.group, dev, [call, n_items, int(k), int(batch_size or 0), int(bool(exclude_self)),
+                                           *rec._exclude_kind(exclude), rec._n_candidates(candidates),
+                                           METHODS.index(method) if method in METHODS else -1])
+    except ValueError as err:
+        raise ValueError("heuristics.recommend / rank_against_all on a row-partitioned graph are collective: every "
+                         "rank must pass the same number of queries, k, method, exclude, exclude_self, batch_size "
+                         "and number of candidates") from err
+    _check_method(method)
+    return dev, rec.candidate_set(candidates, sadj.n_global, dev)
+
+
+def _rank_shard(sadj, method, exclude, exclude_self, cand, dev):
+    n = sadj.n_global
+    e = _exclude_edges(exclude, n, dev)
+    lo, hi = parallel.row_block(n, sadj.rank, sadj.world_size)
+    rowptr, col = rec.shard_exclude_csr(e, lo, hi, n, sadj.local_t)
+    return RankShard(neighbour_table(sadj), method, n, sadj.rank, sadj.world_size, rowptr, col, exclude_self, cand)
+
+
+def _exchange(shard, q, group):
+    """the rank's fp64 partial P and its fp32 block of summed scores"""
+    import torch.distributed as dist
+    P, send = shard.partial(q)
+    recv = torch.empty_like(send)
+    with profiling.span("heuristics: exchange (all_to_all partials)"):
+        dist.all_to_all_single(recv, send, group=group)
+    return P, shard.combine(recv)
+
+
+@torch.no_grad()
+def _recommend_sharded(sadj, nodes, k, method, exclude, exclude_self, batch_size, candidates):
+    import torch.distributed as dist
+    nodes = torch.as_tensor(nodes)
+    dev, cand = _sharded_setup(sadj, 1, nodes.numel(), k, method, exclude, exclude_self, batch_size, candidates)
+    k = rec._check_k(k)
+    nodes = rec._node_ids(nodes, sadj.n_global, "nodes").reshape(-1).to(dev)
+    if cand is not None and cand.numel() == 0:
+        return rec._no_candidates(nodes.numel(), k, dev)
+    shard = _rank_shard(sadj, method, exclude, exclude_self, cand, dev)
+    bs = shard.batch_size(batch_size)
+    R, Q = shard.R, nodes.numel()
+    ids = torch.empty(Q, k, dtype=torch.int64, device=dev)
+    scores = torch.empty(Q, k, dtype=torch.float32, device=dev)
+    for i in range(0, Q, bs):
+        q = nodes[i:i + bs]
+        _, S = _exchange(shard, q, sadj.group)
+        mine_i, mine_s = shard.topk(S, q, k)
+        with profiling.span("heuristics: exchange (all_gather top-k)"):
+            all_i = torch.empty(R * q.numel(), k, dtype=torch.int64, device=dev)
+            all_s = torch.empty(R * q.numel(), k, dtype=torch.float32, device=dev)
+            dist.all_gather_into_tensor(all_i, mine_i, group=sadj.group)
+            dist.all_gather_into_tensor(all_s, mine_s, group=sadj.group)
+        ids[i:i + bs], scores[i:i + bs] = _ops.topk_merge_raw(all_i.view(R, -1, k), all_s.view(R, -1, k), k)
+    return ids, scores
+
+
+@torch.no_grad()
+def _rank_sharded(sadj, edges, method, exclude, exclude_self, batch_size, candidates):
+    import torch.distributed as dist
+    edges = torch.as_tensor(edges)
+    dev, cand = _sharded_setup(sadj, 2, edges.numel(), 0, method, exclude, exclude_self, batch_size, candidates)
+    edges = rec._edge_ids(edges, sadj.n_global).to(dev)
+    if cand is not None and cand.numel() == 0:
+        return torch.ones(edges.size(0), dtype=torch.float32, device=dev)
+    shard = _rank_shard(sadj, method, exclude, exclude_self, cand, dev)
+    bs = shard.batch_size(batch_size)
+    src, tgt = edges[:, 0].contiguous(), edges[:, 1].contiguous()
+    ranks = torch.empty(edges.size(0), dtype=torch.float32, device=dev)
+    for i in range(0, edges.size(0), bs):
+        q, t = src[i:i + bs], tgt[i:i + bs]
+        P, S = _exchange(shard, q, sadj.group)
+        mine = shard.ranker.target_values(P, q, t)
+        with profiling.span("heuristics: exchange (all_gather target partials)"):
+            parts = torch.empty(shard.R * q.numel(), dtype=torch.float64, device=dev)
+            dist.all_gather_into_tensor(parts, mine, group=sadj.group)
+        c = shard.counts(S, q, t, shard.target_scores(parts.view(shard.R, -1)))
+        with profiling.span("heuristics: exchange (all_reduce counts)"):
+            dist.all_reduce(c, group=sadj.group)
+        ranks[i:i + bs] = 0.5 * (c[0].to(torch.float32) + c[1].to(torch.float32)) + 1.0
+    return ranks
+
+
+@torch.no_grad()
+def recommend(adj_t, nodes, k, method, exclude=None, exclude_self=True, batch_size=None, candidates=None):
+    """-> (ids int64 [Q, k], scores fp32 [Q, k]) on the adjacency's device: row q holds the k nodes j with the largest
+    ``method`` heuristic of (nodes[q], j) ('CN', 'AA' or 'RA', the semantics of ``score_edges``, bit for bit), by
+    score descending then id ascending; excluded nodes (and nodes[q] itself when ``exclude_self``) never appear.
+    Every node outside the two-hop set of the query scores exactly +0.0 and is a candidate like any other, so where
+    fewer than k nodes score above 0 the row is filled with score-0 nodes in ascending id order; a row runs short,
+    ending in (-1, -inf), only when fewer than k nodes are left at all.  ``exclude``: None, 'adj' (the stored rows
+    of ``adj_t``) or an int64 [E, 2] tensor of known links (src, dst).  ``batch_size``: queries per chunk (default:
+    a chunk of about 1 GiB); results do not depend on it.  ``candidates``: an int64 tensor of node ids (a set); only
+    those nodes are recommended, as if every other node were an excluded link of every query.  1 <= k <= 1024.  A
+    bad method, k, dtype or shape, an id out of range, a bad exclude or candidate set raises ValueError.  ``adj_t`` a
+    ``parallel.ShardedAdj``: a collective call, every rank passes the same arguments and gets the full result."""
+    if isinstance(adj_t, parallel.ShardedAdj):
+        return _recommend_sharded(adj_t, nodes, k, method, exclude, exclude_self, batch_size, candidates)
+    _check_method(method)
+    k = rec._check_k(k)
+    n = _n_nodes(adj_t)
+    dev = adj_t.csr()[1].device
+    nodes = rec._node_ids(nodes, n, "nodes").reshape(-1).to(dev)
+    cand = rec.candidate_set(candidates, n, dev)
+    e = _exclude_edges(exclude, n, dev)
+    W = n if cand is None else cand.numel()
+    bs = _chunk_rows(batch_size, query_bytes(W))
+    if W == 0:
+        return rec._no_candidates(nodes.numel(), k, dev)
+    rowptr, col = rec.exclude_csr(adj_t, e, n, dev)
+    ranker = Ranker(neighbour_table(adj_t), method, W, cand=cand)
+    Q = nodes.numel()
+    ids = torch.empty(Q, k, dtype=torch.int64, device=dev)
+    scores = torch.empty(Q, k, dtype=torch.float32, device=dev)
+    for i in range(0, Q, bs):
+        q = nodes[i:i + bs]
+        S = _mask(ranker.chunk(q), q, rowptr, col, exclude_self, cand=cand)
+        ids[i:i + bs], scores[i:i + bs], _, _ = _select(S, k, cand=cand)
+    return ids, scores
+
+
+@torch.no_grad()
+def rank_against_all(adj_t, edges, method, exclude=None, exclude_self=True, batch_size=None, candidates=None):
+    """-> fp32 [P]: the filtered rank of each target edges[p, 1] among all nodes (or the ``candidates`` plus the
+    target) for the source edges[p, 0] under the ``method`` heuristic, 1 + (gt + ge) / 2, where gt (ge) counts the
+    candidates j != target that are not excluded and score > (>=) the target.  The target is never excluded.  A
+    target outside the two-hop set of its source scores 0 and gets the mean tie rank among all score-0 candidates --
+    the true filtered rank, and a common case for CN on a sparse graph.  Arguments and errors as ``recommend``;
+    collective on a row-partitioned graph."""
+    if isinstance(adj_t, parallel.ShardedAdj):
+        return _rank_sharded(adj_t, edges, method, exclude, exclude_self, batch_size, candidates)
+    _check_method(method)
+    n = _n_nodes(adj_t)
+    dev = adj_t.csr()[1].device
+    edges = rec._edge_ids(edges, n).to(dev)
+    cand = rec.candidate_set(candidates, n, dev)
+    e = _exclude_edges(exclude, n, dev)
+    W = n if cand is None else cand.numel()
+    bs = _chunk_rows(batch_size, query_bytes(W))
+    if W == 0:
+        return torch.ones(edges.size(0), dtype=torch.float32, device=dev)
+    rowptr, col = rec.exclude_csr(adj_t, e, n, dev)
+    ranker = Ranker(neighbour_table(adj_t), method, W, cand=cand)
+    src, tgt = edges[:, 0].contiguous(), edges[:, 1].contiguous()
+    ranks = torch.empty(edges.size(0), dtype=torch.float32, device=dev)
+    for i in range(0, edges.size(0), bs):
+        q, t = src[i:i + bs], tgt[i:i + bs]
+        S = ranker.chunk(q)
+        ts = ranker.target_values(S, q, t)          # read before the mask: the target is never excluded
+        _, _, gt, ge = _select(_mask(S, q, rowptr, col, exclude_self, cand=cand), 0, t, ts, cand=cand)
+        ranks[i:i + bs] = 0.5 * (gt.to(torch.float32) + ge.to(torch.float32)) + 1.0
+    return ranks

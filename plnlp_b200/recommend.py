@@ -295,16 +295,15 @@ def candidate_slices(cand, bounds):
     return [(at[2 * r], at[2 * r + 1]) for r in range(len(bounds))]
 
 
-def exclude_csr(data, exclude, n, device):
+def exclude_csr(adj, exclude, n, device):
     """the known links to filter, as (rowptr int64 [n + 1], col int32) on the device, or (None, None):
-    ``None``; ``'adj'``: the stored rows of data.adj_t; an int64 [E, 2] edge tensor: row q lists the dst of every
-    edge whose src is q (built with CSRGraph.from_edge_index)"""
+    ``None``; ``'adj'``: the stored rows of the adjacency ``adj``; an int64 [E, 2] edge tensor: row q lists the dst
+    of every edge whose src is q (built with CSRGraph.from_edge_index)"""
     if exclude is None:
         return None, None
     if isinstance(exclude, str):
         if exclude != "adj":
             raise ValueError(f"exclude: expected None, 'adj' or an int64 [E, 2] edge tensor, got {exclude!r}")
-        adj = data.adj_t
         if adj.size(0) != n:
             raise ValueError(f"exclude='adj': the adjacency has {adj.size(0)} rows, the graph {n} nodes")
         st = _ops.structure_of(adj)
@@ -518,7 +517,7 @@ def recommend(model, data, nodes, k, exclude=None, exclude_self=True, batch_size
     h = _encode(model, data)
     n, dev = h.size(0) - 1, h.device
     nodes = _node_ids(nodes, n, "nodes").reshape(-1).to(dev)
-    rowptr, col = exclude_csr(data, exclude, n, dev)
+    rowptr, col = exclude_csr(data.adj_t, exclude, n, dev)
     scorer = _Scorer(model, h, cand=cand)
     bs = int(batch_size) if batch_size else scorer.default_batch_size()
     Q = nodes.numel()
@@ -551,7 +550,7 @@ def rank_against_all(model, data, edges, exclude=None, exclude_self=True, batch_
     h = _encode(model, data)
     n, dev = h.size(0) - 1, h.device
     edges = _edge_ids(edges, n).to(dev)
-    rowptr, col = exclude_csr(data, exclude, n, dev)
+    rowptr, col = exclude_csr(data.adj_t, exclude, n, dev)
     scorer = _Scorer(model, h, cand=cand)
     bs = int(batch_size) if batch_size else scorer.default_batch_size()
     src, tgt = edges[:, 0].contiguous(), edges[:, 1].contiguous()

@@ -14,7 +14,17 @@ JSON line:
     kernel binary-searches the longer list);
   * the agreement with the oracle's rules (oracle/heuristics.py) on a seeded sample of 10 000 test pairs, recomputed
     on the CPU from the raw stored rows of the adjacency: how many are bit-equal, and the largest difference in fp32
-    ulps."""
+    ulps.
+
+With ``--queries Q [--k K]`` it times heuristic recommendation instead (``heuristics.recommend`` with exclude='adj'
+on Q seeded query nodes, and ``heuristics.rank_against_all`` on the first Q (source, target) pairs of the test split)
+and prints one JSON line with: the first call including the table builds (cleaned CSR, transpose, weights) and the
+median of R cached calls (CUDA events); the per-kernel split of one instrumented call of each (plnlp_b200.profiling
+spans: mark, score, mask, select); the marked (two-hop) pairs per query -- the pairs the score kernel intersects,
+against N pairs per query for ``score_edges`` over every (u, j); the time of that pair-by-pair workaround for
+``--pair-queries`` of the queries, timed in the same call; and a bit-for-bit check of a sample of the returned scores
+against ``score_edges``.  ``--partitioned`` (under torchrun; one rank without it) runs the collective calls on
+``parallel.shard_graph`` and checks them against the single-GPU calls on the same rank."""
 import argparse
 import json
 import math
@@ -29,7 +39,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 import bench  # noqa: E402
 from oracle import heuristics as oh  # noqa: E402
-from plnlp_b200 import heuristics  # noqa: E402
+from plnlp_b200 import _ops, heuristics, profiling  # noqa: E402
 from plnlp_b200.graph import CSRGraph  # noqa: E402
 from plnlp_b200.utils import gcn_normalization, get_pos_neg_edges  # noqa: E402
 from recommend_bench import gpu_info, timed  # noqa: E402
@@ -90,19 +100,120 @@ def agreement(adj, edges, method):
             "nonzero_scores": int((want != 0).sum())}
 
 
+_POPCOUNT = None
+
+
+def marked_pairs(table, nodes, chunk=64):
+    """the bits the mark kernel sets for ``nodes`` over all columns: the (query, j) pairs the score kernel
+    intersects"""
+    global _POPCOUNT
+    if _POPCOUNT is None:
+        _POPCOUNT = torch.tensor([bin(i).count("1") for i in range(256)], dtype=torch.int64, device=nodes.device)
+    rr, rc = table.reach()
+    total = 0
+    for i in range(0, nodes.numel(), chunk):
+        bm = _ops.two_hop_mark_raw(table.rowptr, table.col, rr, rc, nodes[i:i + chunk], table.n)
+        total += int(_POPCOUNT[bm.view(torch.uint8).to(torch.int64)].sum())
+    return total
+
+
+def split_of(spans):
+    return {name: {"n": v["n"], "ms": round(v["ms"], 3)} for name, v in sorted(spans.items())}
+
+
+def recommend_main(args, cfg, data, split, dev):
+    import torch.distributed as dist
+    N = cfg["N"]
+    adj = data.adj_t
+    graph = adj
+    if args.partitioned:
+        from plnlp_b200 import parallel
+        if "RANK" not in os.environ:
+            os.environ.update(RANK="0", WORLD_SIZE="1", LOCAL_RANK="0", MASTER_ADDR="127.0.0.1", MASTER_PORT="29541")
+        dist.init_process_group("nccl", device_id=dev)
+        graph = parallel.shard_graph(adj, dist.get_rank(), dist.get_world_size(), CSRGraph, symmetric=True)
+    g = torch.Generator(device=dev).manual_seed(7)
+    nodes = torch.randint(0, N, (args.queries,), generator=g, device=dev)
+    pos, _ = get_pos_neg_edges("test", split, device=dev)
+    edges = pos[:args.queries].contiguous()
+    m, k = args.method, args.k
+    rec = lambda: heuristics.recommend(graph, nodes, k, m, "adj")           # noqa: E731
+    rank = lambda: heuristics.rank_against_all(graph, edges, m, "adj")      # noqa: E731
+    res = {"workload": cfg["name"], "gpu": gpu_info(), "method": m, "N": N, "queries": args.queries, "k": k,
+           "exclude": "adj", "partitioned": bool(args.partitioned),
+           "ranks": dist.get_world_size() if args.partitioned else 1}
+    for name, fn in (("recommend", rec), ("rank_against_all", rank)):
+        heuristics._CACHE.clear()
+        first, out = timed(fn, 1)
+        times = [timed(fn, 1)[0] for _ in range(args.reps)]
+        profiling.enable()
+        fn()
+        spans = profiling.disable()
+        res[name] = {"first_call_ms_with_table_builds": round(first, 2), "ms_median": round(float(np.median(times)), 2),
+                     "ms_all": [round(t, 2) for t in times],
+                     "ms_per_query": round(float(np.median(times)) / args.queries, 4), "split": split_of(spans)}
+        res[name + "_out"] = out
+    ids, scores = res.pop("recommend_out")
+    ranks = res.pop("rank_against_all_out")
+    res["rank_against_all"]["mrr"] = round(float((1.0 / ranks).mean()), 5)
+    res["rank_against_all"]["targets_scoring_0"] = int((heuristics.score_edges(graph, edges, m) == 0).sum())
+    table = heuristics.neighbour_table(adj)
+    marked = marked_pairs(table, nodes)
+    res["two_hop"] = {"marked_pairs_per_query": round(marked / args.queries, 1), "all_pairs_per_query": N,
+                      "share": round(marked / args.queries / N, 6)}
+    # the returned scores against score_edges, bit for bit
+    sample = min(args.queries, 64)
+    live = ids[:sample] >= 0
+    pairs = torch.stack([nodes[:sample, None].expand(-1, k)[live], ids[:sample][live]], 1)
+    want = heuristics.score_edges(graph, pairs, m)
+    res["score_edges_check"] = {"pairs": int(pairs.size(0)),
+                                "bit_equal": int((want.view(torch.int32) == scores[:sample][live].view(torch.int32)).sum())}
+    if args.partitioned:
+        si, ss = heuristics.recommend(adj, nodes, k, m, "adj")
+        sr = heuristics.rank_against_all(adj, edges, m, "adj")
+        res["single_gpu_check"] = {"ids_equal": bool(torch.equal(si, ids)), "scores_equal": bool(torch.equal(ss, scores)),
+                                   "ranks_equal": bool(torch.equal(sr, ranks))}
+    else:
+        # the pair-by-pair workaround: score_edges over every (u, j), then the same top-k select, for a few queries
+        Qp = min(args.pair_queries, args.queries)
+        j = torch.arange(N, device=dev)
+
+        def pairwise():
+            out = []
+            for u in nodes[:Qp].tolist():
+                S = heuristics.score_edges(adj, torch.stack([torch.full_like(j, u), j], 1), m).reshape(1, N)
+                out.append(_ops.topk_rows_raw(S, k)[0])
+            return out
+        pairwise()
+        ms, _ = timed(pairwise, 1)
+        res["pairwise_workaround"] = {"queries": Qp, "ms": round(ms, 2), "ms_per_query": round(ms / Qp, 3),
+                                      "note": "score_edges over all N pairs plus the select, no exclusion mask"}
+    if not args.partitioned or dist.get_rank() == 0:
+        print(json.dumps(res))
+    if args.partitioned:
+        dist.destroy_process_group()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("workload", nargs="?", default="citation2", choices=["citation2", "collab", "ddi"])
     ap.add_argument("--method", default="CN", choices=list(heuristics.METHODS))
     ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--queries", type=int, default=0, help="time recommend / rank_against_all on this many queries")
+    ap.add_argument("--k", type=int, default=100)
+    ap.add_argument("--pair-queries", type=int, default=4)
+    ap.add_argument("--partitioned", action="store_true")
     args = ap.parse_args()
-    dev = torch.device("cuda")
+    dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", 0)))
+    torch.cuda.set_device(dev)
     cfg = dict(bench.WORKLOADS[args.workload])
     torch.manual_seed(0)
     data, split = bench.build_workload(cfg, dev, CSRGraph, gcn_normalization)
     N = cfg["N"]
     eval_split, metric = build_splits(args.workload, N, dev)
     split.update(eval_split)
+    if args.queries > 0:
+        return recommend_main(args, cfg, data, split, dev)
     adj = data.adj_t
 
     builds = []
