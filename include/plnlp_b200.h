@@ -475,6 +475,27 @@ int plnlp_two_hop_score_f64(const int64_t* rowptr, const int32_t* col, int64_t n
                             const int64_t* nodes, int64_t Qc, int64_t col0, int64_t W, const int64_t* cand,
                             const uint32_t* bitmap, double* s, int64_t lds, void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * Path-based link scores (plnlp_b200/paths.py; csrc/propagate.cu): one hop of Katz or Personalized PageRank for a
+ * block of B source columns, B in {32, 64, 128, 256}.  x [n, B] fp32, node-major, row stride ldx >= B; for every
+ * output row j of [r0, r0 + rows):
+ *   y[j - r0, c] = fp32(cm * s + (src[c] == j ? ba : 0)),  s = sum over the entries w of row j of weight[w] * x[w, c]
+ * (weight fp64 [n], or 1 per entry when NULL), with cm / ba the fp64 values whose bit patterns are c_bits / b_bits.
+ * Products, sums, the multiply and the add are fp64 rounded to nearest (no contraction); one rounding to fp32.
+ * The rows are walked through an SpMM work plan over their entries (item_ptr [n_items + 1], item_row, item_slot,
+ * fix_ptr / fix_row for the n_fix split rows, as plnlp_spmm_csr_f32); an item's entries are summed in order, a split
+ * row's partials (partial fp64 [n_partial, B]) in item order, so every bit depends on the plan and the inputs only.
+ * src int64 [B]: the source node of each column, -1 for a padding column.  Every x and weight must be >= 0.
+ * live_in uint8 [n] or NULL: 0 promises an all-zero row of x, which is then not read (this changes no bit).
+ * live_out uint8 [rows] or NULL: 1 where the output row has a non-zero entry, else 0.  y [rows, B], row stride
+ * ldy >= B.  x, y, ldx and ldy aligned to min(B / 32, 4) floats (PLNLP_E_ALIGN).  Run-to-run deterministic.
+ * ------------------------------------------------------------------------------------ */
+int plnlp_propagate_f32(const int32_t* item_ptr, const int32_t* item_row, const int32_t* item_slot, int64_t n_items,
+                        const int32_t* col, const int32_t* fix_ptr, const int32_t* fix_row, int64_t n_fix,
+                        double* partial, const double* weight, const float* x, int64_t ldx, const int64_t* src,
+                        int64_t B, uint64_t c_bits, uint64_t b_bits, const uint8_t* live_in, uint8_t* live_out,
+                        int64_t r0, int64_t rows, float* y, int64_t ldy, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

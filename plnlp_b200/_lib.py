@@ -84,6 +84,8 @@ SIGNATURES = {
     "plnlp_two_hop_mark": (c_int, [_P, _P, _P, _P, _L, _P, _P, _L, _L, _L, _P, _P, _P]),
     "plnlp_two_hop_score_f32": (c_int, [_P, _P, _L, _L, _P, _P, _L, _L, _L, _P, _P, _P, _L, _P]),
     "plnlp_two_hop_score_f64": (c_int, [_P, _P, _L, _L, _P, _P, _L, _L, _L, _P, _P, _P, _L, _P]),
+    "plnlp_propagate_f32": (c_int, [_P, _P, _P, _L, _P, _P, _P, _L, _P, _P, _P, _L, _P, _L, _U, _U, _P, _P, _L, _L, _P,
+                                    _L, _P]),
 }
 
 _ERRORS = {-1: "required pointer is NULL", -2: "bad size", -3: "misaligned pointer / leading dimension",

@@ -1378,3 +1378,40 @@ def two_hop_score_raw(rowptr, col, weight, nodes, bitmap, W, col0=0, cand=None, 
                 ptr(None if weight is None else weight.contiguous()), ptr(nodes), Qc, int(col0), int(W), ptr(cand),
                 ptr(bitmap.contiguous()), ptr(s), W, stream()), "plnlp_two_hop_score")
     return s
+
+
+def _f64_bits(v):
+    import struct
+    return struct.unpack("<Q", struct.pack("<d", float(v)))[0]
+
+
+def propagate_raw(plan, weight, x, src, c, b, live_in=None, r0=0, y=None, live_out=None):
+    """one hop of the path scores (paths.py): for every row j of [r0, r0 + plan.n_rows), y[j - r0, a] =
+    fp32(c * sum over the row's entries w of weight[w] * x[w, a] + (b if src[a] == j else 0)) in fp64, summed in the
+    order of ``plan`` (graph.build_plan over the rows).  x fp32 [n, B] node-major (B in 32, 64, 128, 256, row stride
+    free), weight fp64 [n] or None (1), src int64 [B] (-1: padding column), live_in uint8 [n] or None (every row
+    read).  -> (y fp32 [rows, B], live_out uint8 [rows]); ``y`` / ``live_out`` may be given (y's rows contiguous)."""
+    lib = _lib.load()
+    B = x.size(1)
+    rows = plan.n_rows
+    if x.dtype != torch.float32 or x.stride(1) != 1 or src.dtype != torch.int64 or src.numel() != B:
+        raise RuntimeError("propagate_raw: x must be fp32 [n, B] with unit column stride and src int64 [B]")
+    if weight is not None and weight.dtype != torch.float64:
+        raise RuntimeError("propagate_raw: weight must be fp64")
+    if live_in is not None and (live_in.dtype != torch.uint8 or live_in.numel() < x.size(0)):
+        raise RuntimeError("propagate_raw: live_in must be uint8 [n]")
+    if y is None:
+        y = torch.empty(rows, B, dtype=torch.float32, device=x.device)
+    if live_out is None:
+        live_out = torch.empty(rows, dtype=torch.uint8, device=x.device)
+    partial = None
+    if plan.n_fix:
+        partial = workspace.get("propagate", plan.n_partial * B * 8, x.device).view(torch.float64)
+    with profiling.span(f"propagate_f32 B={B}", 0, 0):
+        check(lib.plnlp_propagate_f32(ptr(plan.item_ptr), ptr(plan.item_row), ptr(plan.item_slot), plan.n_items,
+                                      ptr(plan.col), ptr(plan.fix_ptr), ptr(plan.fix_row), plan.n_fix, ptr(partial),
+                                      ptr(None if weight is None else weight.contiguous()), ptr(x), x.stride(0),
+                                      ptr(src.contiguous()), B, _f64_bits(c), _f64_bits(b), ptr(live_in),
+                                      ptr(live_out), int(r0), rows, ptr(y), y.stride(0), stream()),
+              "plnlp_propagate_f32")
+    return y, live_out

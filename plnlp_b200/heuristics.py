@@ -40,8 +40,16 @@ does: rank r computes the fp64 partial of every column over w in [lo, hi), sends
 sharded mask, select and merge follow.  CN is exact and R = 1 is bit-identical to one GPU; AA and RA lie within one
 fp32 ulp of one GPU (and, at R >= 3, may differ by an ulp from the partitioned ``score_edges``, whose all-reduce
 sums in another order).  ``RankShard`` is the per-rank step, with no collective.
+
+The path-based scores Katz and Personalized PageRank (``Katz``, ``PPR``, ``PATH_METHODS``) go through the same four
+calls and are run by paths.py, which documents their semantics.
 """
 from __future__ import annotations
+
+import math
+import numbers
+from dataclasses import dataclass
+from typing import ClassVar
 
 import torch
 
@@ -50,6 +58,65 @@ from . import recommend as rec
 from .utils import evaluate_hits, evaluate_mrr, get_pos_neg_edges
 
 METHODS = ("CN", "AA", "RA")
+PATH_METHODS = ("Katz", "PPR")         # path-based scores, run by paths.py; the strings mean the default parameters
+PATH_CODES = {"Katz": 10, "PPR": 11}   # their method words in the collective argument check
+MAX_KATZ_HOPS = 32
+MAX_PPR_ITERS = 1000
+
+
+def _int_param(v, name, hi):
+    if isinstance(v, bool) or not isinstance(v, numbers.Integral) or not 1 <= int(v) <= hi:
+        raise ValueError(f"{name} must be an integer in [1, {hi}], got {v!r}")
+    return int(v)
+
+
+def _real_param(v, name):
+    if isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(float(v)):
+        raise ValueError(f"{name} must be a finite real number, got {v!r}")
+    return float(v)
+
+
+@dataclass(frozen=True)
+class Katz:
+    """Katz index truncated at ``hops`` = L: sum over l = 1 .. L of beta^l * (number of length-l walks from u to v
+    along N).  beta finite and > 0, 1 <= hops <= MAX_KATZ_HOPS; anything else raises ValueError."""
+    beta: float = 0.005
+    hops: int = 3
+    name: ClassVar[str] = "Katz"
+
+    def __post_init__(self):
+        beta = _real_param(self.beta, "Katz beta")
+        if not beta > 0.0:
+            raise ValueError(f"Katz beta must be > 0, got {self.beta!r}")
+        object.__setattr__(self, "beta", beta)
+        object.__setattr__(self, "hops", _int_param(self.hops, "Katz hops", MAX_KATZ_HOPS))
+
+
+@dataclass(frozen=True)
+class PPR:
+    """Personalized PageRank of v for the source u after ``iters`` = T power iterations x <- (1 - alpha) P^T x +
+    alpha e_u from x = e_u, P the row-stochastic walk on N (a walker at a node without neighbours is dropped).
+    0 < alpha < 1, 1 <= iters <= MAX_PPR_ITERS; anything else raises ValueError."""
+    alpha: float = 0.15
+    iters: int = 30
+    name: ClassVar[str] = "PPR"
+
+    def __post_init__(self):
+        alpha = _real_param(self.alpha, "PPR alpha")
+        if not 0.0 < alpha < 1.0:
+            raise ValueError(f"PPR alpha must lie in (0, 1), got {self.alpha!r}")
+        object.__setattr__(self, "alpha", alpha)
+        object.__setattr__(self, "iters", _int_param(self.iters, "PPR iters", MAX_PPR_ITERS))
+
+
+def path_method(method):
+    """the ``Katz`` / ``PPR`` parameters of a path method ('Katz', 'PPR' or an instance), or None for any other
+    method"""
+    if isinstance(method, (Katz, PPR)):
+        return method
+    if isinstance(method, str) and method in PATH_METHODS:
+        return Katz() if method == "Katz" else PPR()
+    return None
 
 
 def clean_csr(row, col, n):
@@ -198,7 +265,12 @@ def score_edges(adj_t, edges, method, batch_size=None):
     docstring) of every pair edges[p] = (u, v), an int64 [P, 2] tensor of node ids in [0, n).  ``batch_size``: pairs
     per kernel launch (default: all).  Raises ValueError for another method, dtype or shape, or ids out of range.
     ``adj_t`` a ``parallel.ShardedAdj``: a collective call, every rank passes the same arguments and gets the full
-    result."""
+    result.  ``method`` may also be a path method, 'Katz', 'PPR', ``Katz(...)`` or ``PPR(...)`` (paths.py); then
+    ``batch_size`` is the number of sources propagated together (see ``recommend``)."""
+    pm = path_method(method)
+    if pm is not None:
+        from . import paths
+        return paths.score_edges(adj_t, edges, pm, batch_size)
     if isinstance(adj_t, parallel.ShardedAdj):
         return _score_sharded(adj_t, edges, method, batch_size)
     _check_method(method)
@@ -491,7 +563,16 @@ def recommend(adj_t, nodes, k, method, exclude=None, exclude_self=True, batch_si
     a chunk of about 1 GiB); results do not depend on it.  ``candidates``: an int64 tensor of node ids (a set); only
     those nodes are recommended, as if every other node were an excluded link of every query.  1 <= k <= 1024.  A
     bad method, k, dtype or shape, an id out of range, a bad exclude or candidate set raises ValueError.  ``adj_t`` a
-    ``parallel.ShardedAdj``: a collective call, every rank passes the same arguments and gets the full result."""
+    ``parallel.ShardedAdj``: a collective call, every rank passes the same arguments and gets the full result.
+
+    Path methods ('Katz', 'PPR', ``Katz(...)``, ``PPR(...)``; paths.py): the query's column of the propagated state
+    is its score row, a node the walks never reach scores +0.0, and the rules above are unchanged.  ``batch_size``
+    is then the number of queries propagated together, rounded up to 32, 64, 128 or 256 (default:
+    as many as fit ``paths.PATH_BYTES``); results do not depend on it."""
+    pm = path_method(method)
+    if pm is not None:
+        from . import paths
+        return paths.recommend(adj_t, nodes, k, pm, exclude, exclude_self, batch_size, candidates)
     if isinstance(adj_t, parallel.ShardedAdj):
         return _recommend_sharded(adj_t, nodes, k, method, exclude, exclude_self, batch_size, candidates)
     _check_method(method)
@@ -524,7 +605,11 @@ def rank_against_all(adj_t, edges, method, exclude=None, exclude_self=True, batc
     candidates j != target that are not excluded and score > (>=) the target.  The target is never excluded.  A
     target outside the two-hop set of its source scores 0 and gets the mean tie rank among all score-0 candidates --
     the true filtered rank, and a common case for CN on a sparse graph.  Arguments and errors as ``recommend``;
-    collective on a row-partitioned graph."""
+    collective on a row-partitioned graph.  Path methods as in ``recommend``."""
+    pm = path_method(method)
+    if pm is not None:
+        from . import paths
+        return paths.rank_against_all(adj_t, edges, pm, exclude, exclude_self, batch_size, candidates)
     if isinstance(adj_t, parallel.ShardedAdj):
         return _rank_sharded(adj_t, edges, method, exclude, exclude_self, batch_size, candidates)
     _check_method(method)

@@ -24,7 +24,16 @@ spans: mark, score, mask, select); the marked (two-hop) pairs per query -- the p
 against N pairs per query for ``score_edges`` over every (u, j); the time of that pair-by-pair workaround for
 ``--pair-queries`` of the queries, timed in the same call; and a bit-for-bit check of a sample of the returned scores
 against ``score_edges``.  ``--partitioned`` (under torchrun; one rank without it) runs the collective calls on
-``parallel.shard_graph`` and checks them against the single-GPU calls on the same rank."""
+``parallel.shard_graph`` and checks them against the single-GPU calls on the same rank.
+
+With ``--method Katz|PPR`` (``--beta/--hops`` or ``--alpha/--iters``) it times the path-based scores (paths.py) and
+prints one JSON line with: per hop of one block of 256 sources, the kernel time (CUDA events), the live-row fraction
+of the state it reads, the bytes it gathers (the live rows' state entries, every column index and live byte, the
+output) and those bytes/s against the 7.7 TB/s data-sheet peak; the eval-split pairs/s of ``score_edges`` over the
+pairs of ``--sources`` distinct test sources (a labelled subset; the full-split time is extrapolated linearly and
+labelled so); ``recommend`` per-query time on 256 queries with its kernel split; and the agreement of a sample of
+scores with the fp64 series computed on the CPU with scipy from the cleaned reach table.  ``--partitioned`` runs the
+collective calls as above and checks them against one GPU."""
 import argparse
 import json
 import math
@@ -194,10 +203,116 @@ def recommend_main(args, cfg, data, split, dev):
         dist.destroy_process_group()
 
 
+PEAK_BYTES_PER_S = 7.7e12      # HBM3e, NVIDIA HGX B200 data sheet, one GPU
+
+
+def fp64_series(table_rowptr, table_col, inv_deg, method, sources):
+    """fp64 [N, S] on the CPU (scipy): the truncated series of ``method`` for the sources, hop by hop from the
+    cleaned reach rows R(j), with no fp32 rounding"""
+    import scipy.sparse as sp
+    from plnlp_b200 import paths
+    rp, col = table_rowptr.cpu().numpy(), table_col.cpu().numpy()
+    n = rp.size - 1
+    Rm = sp.csr_matrix((np.ones(col.size), col, rp), shape=(n, n))
+    wt = inv_deg.cpu().numpy()[:, None]
+    E = np.zeros((n, len(sources)))
+    E[np.asarray(sources), np.arange(len(sources))] = 1.0
+    x = E.copy()
+    for c, b, weighted in paths.hops(method):
+        x = c * (Rm @ (wt * x if weighted else x)) + b * E
+    return x
+
+
+def path_main(args, cfg, data, split, dev):
+    import torch.distributed as dist
+    from plnlp_b200 import parallel, paths
+    N, adj = cfg["N"], data.adj_t
+    m = heuristics.Katz(args.beta, args.hops) if args.method == "Katz" else heuristics.PPR(args.alpha, args.iters)
+    graph = adj
+    if args.partitioned:
+        if "RANK" not in os.environ:
+            os.environ.update(RANK="0", WORLD_SIZE="1", LOCAL_RANK="0", MASTER_ADDR="127.0.0.1", MASTER_PORT="29541")
+        dist.init_process_group("nccl", device_id=dev)
+        graph = parallel.shard_graph(adj, dist.get_rank(), dist.get_world_size(), CSRGraph, symmetric=True)
+    res = {"workload": cfg["name"], "gpu": gpu_info(), "method": repr(m), "N": N, "partitioned": bool(args.partitioned),
+           "ranks": dist.get_world_size() if args.partitioned else 1}
+    ms, shard = timed(lambda: paths.path_shard(adj).plan(), 1)
+    shard = paths.path_shard(adj)
+    res["table"] = {"build_ms_first": round(ms, 2), "reach_entries": int(shard.col.numel())}
+    pos, neg = get_pos_neg_edges("test", split, device=dev)
+    e_all = torch.cat([pos, neg.reshape(-1, 2)])
+    us = torch.unique(e_all[:, 0])
+    # per hop of one block of 256 sources
+    B = 256
+    src = us[:B].contiguous()
+    x, live = shard.start(src)
+    nnz = int(shard.col.numel())
+    per_hop = []
+    for h, (c, b, w) in enumerate(paths.hops(m)):
+        shard.hop(x, live, src, c, b, w)                                   # warm-up of this hop's inputs
+        ms, (y, lv) = timed(lambda: shard.hop(x, live, src, c, b, w), 1)
+        live_entries = int(live[shard.col.long()].sum())
+        nbytes = live_entries * B * 4 + nnz * 5 + N * B * 4 + N
+        per_hop.append({"hop": h + 1, "ms": round(ms, 3), "live_row_fraction_in": round(float(live.float().mean()), 5),
+                        "gathered_GB": round(nbytes / 1e9, 3), "GB_per_s": round(nbytes / ms / 1e6, 1),
+                        "share_of_7.7TB_per_s": round(nbytes / ms / 1e-3 / PEAK_BYTES_PER_S, 3)})
+        x, live = y, lv
+    res["hops_B256"] = per_hop
+    res["block_B256_ms"] = round(sum(h["ms"] for h in per_hop), 2)
+    # eval split: the pairs of a subset of the distinct test sources
+    S = min(args.sources, us.numel())
+    keep = torch.isin(e_all[:, 0], us[:S])
+    e = e_all[keep].contiguous()
+    heuristics.score_edges(graph, e[:1000], m)
+    times = [timed(lambda: heuristics.score_edges(graph, e, m), 1)[0] for _ in range(args.reps)]
+    ms = float(np.median(times))
+    res["eval_split_subset"] = {"subset": f"pairs of the first {S} of {us.numel()} distinct test sources",
+                                "sources": S, "pairs": int(e.size(0)), "ms_median": round(ms, 1),
+                                "pairs_per_s": round(e.size(0) / ms * 1e3),
+                                "extrapolated_full_split_s": round(ms * us.numel() / S / 1e3, 1),
+                                "extrapolation": "linear in distinct sources (blocks of 256); not measured"}
+    out = heuristics.score_edges(graph, e, m)
+    # recommend on 256 queries
+    g = torch.Generator(device=dev).manual_seed(7)
+    nodes = torch.randint(0, N, (256,), generator=g, device=dev)
+    fn = lambda: heuristics.recommend(graph, nodes, args.k, m, "adj")      # noqa: E731
+    fn()
+    times = [timed(fn, 1)[0] for _ in range(args.reps)]
+    profiling.enable()
+    ids, sc = fn()
+    spans = profiling.disable()
+    res["recommend"] = {"queries": 256, "k": args.k, "exclude": "adj", "ms_median": round(float(np.median(times)), 2),
+                        "ms_per_query": round(float(np.median(times)) / 256, 4), "split": split_of(spans)}
+    if args.partitioned:
+        si, ss = heuristics.recommend(adj, nodes, args.k, m, "adj")
+        res["single_gpu_check"] = {"ids_equal": bool(torch.equal(si, ids)), "scores_equal": bool(torch.equal(ss, sc)),
+                                   "scores_edges_equal": bool(torch.equal(heuristics.score_edges(adj, e, m), out))}
+    # oracle sample: the fp64 series for 8 sources against the kernel's scores of their pairs
+    pick = us[:S][torch.randperm(S, generator=torch.Generator().manual_seed(5))[:8].to(dev)].sort().values
+    ref = fp64_series(shard.rowptr, shard.col, shard.inv_deg, m, pick.cpu().numpy())
+    sel = torch.isin(e[:, 0], pick)
+    pe, got = e[sel].cpu(), out[sel].cpu().double().numpy()
+    want = ref[pe[:, 1].numpy(), torch.searchsorted(pick.cpu(), pe[:, 0]).numpy()]
+    rel = np.abs(got - want) / np.maximum(np.abs(want), 1e-300)
+    res["oracle_sample"] = {"pairs": int(pe.size(0)), "sources": 8, "within_1e-5_rel": int((rel <= 1e-5).sum()),
+                            "max_rel_err": float(rel.max()) if rel.size else 0.0,
+                            "nonzero": int((want > 0).sum())}
+    res["gpu_after"] = gpu_info()
+    if not args.partitioned or dist.get_rank() == 0:
+        print(json.dumps(res))
+    if args.partitioned:
+        dist.destroy_process_group()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("workload", nargs="?", default="citation2", choices=["citation2", "collab", "ddi"])
-    ap.add_argument("--method", default="CN", choices=list(heuristics.METHODS))
+    ap.add_argument("--method", default="CN", choices=list(heuristics.METHODS) + list(heuristics.PATH_METHODS))
+    ap.add_argument("--beta", type=float, default=0.005)
+    ap.add_argument("--hops", type=int, default=3)
+    ap.add_argument("--alpha", type=float, default=0.15)
+    ap.add_argument("--iters", type=int, default=30)
+    ap.add_argument("--sources", type=int, default=2048, help="path methods: distinct test sources to time")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--queries", type=int, default=0, help="time recommend / rank_against_all on this many queries")
     ap.add_argument("--k", type=int, default=100)
@@ -212,6 +327,8 @@ def main():
     N = cfg["N"]
     eval_split, metric = build_splits(args.workload, N, dev)
     split.update(eval_split)
+    if args.method in heuristics.PATH_METHODS:
+        return path_main(args, cfg, data, split, dev)
     if args.queries > 0:
         return recommend_main(args, cfg, data, split, dev)
     adj = data.adj_t
