@@ -450,10 +450,18 @@ int plnlp_subset_plan_fill(const int64_t* rowptr, const int64_t* rows, int64_t T
  * Allocation, the non-learned baselines of the OGB link-prediction tables.  rowptr int64 [n + 1] / col int32 [nnz]:
  * a cleaned CSR (every row sorted, distinct, without its diagonal entry).  out[p] (fp64) = the sum over the common
  * neighbours w of rows edges[p, 0] and edges[p, 1] of weight[w] (fp64 [n]), or their count when weight is NULL.
- * edges int64 [P, 2] with ids in [0, n).  Run-to-run deterministic.
+ * edges int64 [P, 2] with ids in [-1, n); a pair with a negative id has no common neighbour.  Run-to-run
+ * deterministic.
  * ------------------------------------------------------------------------------------ */
 int plnlp_link_heuristic_f64(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz, const double* weight,
                              const int64_t* edges, int64_t P, double* out, void* stream);
+/* Common-neighbour lists (plnlp_b200/heuristics.py common_neighbour_lists, the NCN predictor): col_out int32
+ * [out_ptr[P]] receives the common neighbours of rows edges[p, 0] and edges[p, 1] of the same cleaned CSR at
+ * col_out[out_ptr[p] .. out_ptr[p + 1]), in ascending id order.  out_ptr int64 [P + 1]: out_ptr[0] = 0 and
+ * out_ptr[p + 1] - out_ptr[p] = the CN count plnlp_link_heuristic_f64 gives the pair.  Ids in [-1, n) as above. */
+int plnlp_common_neighbour_list(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz,
+                                const int64_t* edges, int64_t P, const int64_t* out_ptr, int32_t* col_out,
+                                void* stream);
 /* Heuristic recommendation over all nodes (plnlp_b200/heuristics.py recommend / rank_against_all): a chunk of Qc
  * query nodes against W candidate columns, the nodes [col0, col0 + W) or, with cand != NULL (strictly ascending
  * global ids, col0 must then be 0, else PLNLP_E_UNSUPPORTED), the nodes cand[0 .. W).

@@ -81,6 +81,7 @@ SIGNATURES = {
     "plnlp_random_walk": (c_int, [_P, _P, _P, _L, _I, _P, _U, _P, _P]),
     "plnlp_walk_pairs": (c_int, [_P, _L, _I, _P, _P, _P, _P]),
     "plnlp_link_heuristic_f64": (c_int, [_P, _P, _L, _L, _P, _P, _L, _P, _P]),
+    "plnlp_common_neighbour_list": (c_int, [_P, _P, _L, _L, _P, _L, _P, _P, _P]),
     "plnlp_two_hop_mark": (c_int, [_P, _P, _P, _P, _L, _P, _P, _L, _L, _L, _P, _P, _P]),
     "plnlp_two_hop_score_f32": (c_int, [_P, _P, _L, _L, _P, _P, _L, _L, _L, _P, _P, _P, _L, _P]),
     "plnlp_two_hop_score_f64": (c_int, [_P, _P, _L, _L, _P, _P, _L, _L, _L, _P, _P, _P, _L, _P]),

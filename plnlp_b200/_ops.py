@@ -1312,9 +1312,9 @@ def topk_merge_raw(ids_in, scores_in, k):
 
 
 def link_heuristic_raw(rowptr, col, weight, edges):
-    """fp64 [P]: for every pair edges[p] = (u, v) (int64 [P, 2], ids in [0, n)) the sum of ``weight[w]`` (fp64 [n])
-    over the common neighbours w of rows u and v of the cleaned CSR (rowptr int64 [n + 1], col int32), or their count
-    when ``weight`` is None (heuristics.py)"""
+    """fp64 [P]: for every pair edges[p] = (u, v) (int64 [P, 2], ids in [-1, n); a pair with a negative id has no
+    common neighbour and gives 0) the sum of ``weight[w]`` (fp64 [n]) over the common neighbours w of rows u and v of
+    the cleaned CSR (rowptr int64 [n + 1], col int32), or their count when ``weight`` is None (heuristics.py)"""
     lib = _lib.load()
     if rowptr.dtype != torch.int64 or col.dtype != torch.int32 or edges.dtype != torch.int64:
         raise RuntimeError("link_heuristic_raw: rowptr and edges must be int64, col int32")
@@ -1327,6 +1327,82 @@ def link_heuristic_raw(rowptr, col, weight, edges):
                                            col.numel(), ptr(None if weight is None else weight.contiguous()),
                                            ptr(edges.contiguous()), P, ptr(out), stream()), "plnlp_link_heuristic_f64")
     return out
+
+
+def common_neighbour_list_raw(rowptr, col, edges, out_ptr):
+    """int32 [out_ptr[-1]]: the common neighbours of every pair edges[p] (int64 [P, 2], ids in [-1, n); a negative id
+    has none) in rows of the cleaned CSR (rowptr int64 [n + 1], col int32), ascending, at [out_ptr[p], out_ptr[p + 1])
+    -- ``out_ptr`` int64 [P + 1] the running sum of the ``link_heuristic_raw`` counts (heuristics.py)"""
+    lib = _lib.load()
+    if rowptr.dtype != torch.int64 or col.dtype != torch.int32 or edges.dtype != torch.int64 \
+            or out_ptr.dtype != torch.int64:
+        raise RuntimeError("common_neighbour_list_raw: rowptr, edges and out_ptr must be int64, col int32")
+    P = edges.size(0)
+    if out_ptr.numel() != P + 1:
+        raise RuntimeError("common_neighbour_list_raw: out_ptr must have P + 1 entries")
+    total = int(out_ptr[-1])
+    out = torch.empty(total, dtype=torch.int32, device=edges.device)
+    if total == 0:
+        return out
+    with profiling.span("common_neighbour_list", P * 16 + total * 4, 0):
+        check(lib.plnlp_common_neighbour_list(ptr(rowptr.contiguous()), ptr(col.contiguous()), rowptr.numel() - 1,
+                                              col.numel(), ptr(edges.contiguous()), P, ptr(out_ptr.contiguous()),
+                                              ptr(out), stream()), "plnlp_common_neighbour_list")
+    return out
+
+
+CN_CHUNK = 256      # entries of a common-neighbour list per SpMM work item: fixes the order of every sum
+
+
+def _cn_plan(rowptr, col, n_rows, n_cols):
+    from .graph import build_plan
+    return build_plan(rowptr, col, None, n_rows, n_cols, chunk=CN_CHUNK)
+
+
+class CommonNeighbourSum(torch.autograd.Function):
+    """c[p] = sum of h[w] over w in col[rowptr[p] .. rowptr[p + 1]) (the NCN predictor's common-neighbour term): the
+    SpMM kernel with the P x N 0/1 matrix of the lists, planned per call at the fixed chunk ``CN_CHUNK`` so every bit
+    of c depends on the list and h only (not on the batch).  Backward: C^T g on the transposed plan (entries sorted by
+    (col, row)), built only when h needs a gradient -- deterministic, no atomics."""
+
+    @staticmethod
+    def forward(ctx, h, rowptr, col):
+        P, n = rowptr.numel() - 1, h.size(0)
+        ctx.save_for_backward(rowptr, col)
+        ctx.n = n
+        if col.numel() == 0:
+            return torch.zeros(P, h.size(1), dtype=torch.float32, device=h.device)
+        with profiling.span("torch: common-neighbour SpMM plan"):
+            plan = _cn_plan(rowptr, col, P, n)
+        with profiling.span("NCN: common-neighbour SpMM forward"):
+            return spmm_raw(plan, h, use_val=False, div_rows=False)
+
+    @staticmethod
+    def backward(ctx, g):
+        rowptr, col = ctx.saved_tensors
+        P, n = rowptr.numel() - 1, ctx.n
+        if not ctx.needs_input_grad[0]:
+            return None, None, None
+        if col.numel() == 0:
+            return torch.zeros(n, g.size(1), dtype=torch.float32, device=g.device), None, None
+        with profiling.span("torch: transposed common-neighbour SpMM plan"):
+            c = col.to(torch.int64)
+            row = torch.repeat_interleave(torch.arange(P, device=c.device), rowptr[1:] - rowptr[:-1],
+                                          output_size=c.numel())
+            perm = torch.argsort(c * P + row, stable=True)
+            t_rowptr = torch.zeros(n + 1, dtype=torch.int64, device=c.device)
+            t_rowptr[1:] = torch.cumsum(torch.bincount(c, minlength=n), 0)
+            plan = _cn_plan(t_rowptr, row[perm], n, P)
+        with profiling.span("NCN: common-neighbour SpMM backward (C^T g)"):
+            return spmm_raw(plan, _rowmajor(g), use_val=False, div_rows=False), None, None
+
+
+def common_neighbour_sum(h, cn):
+    """``CommonNeighbourSum`` of h [N, H] over the lists ``cn = (rowptr int64 [P + 1], col)`` (col: rows of h)"""
+    rowptr, col = cn
+    if rowptr.dtype != torch.int64 or rowptr.dim() != 1 or col.dim() != 1:
+        raise RuntimeError("common_neighbour_sum: cn must be (rowptr int64 [P + 1], col [nnz])")
+    return CommonNeighbourSum.apply(_rowmajor(h), rowptr, col)
 
 
 def _two_hop_args(rowptr, col, nodes, W, col0, cand):

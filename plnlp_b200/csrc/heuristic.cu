@@ -26,13 +26,16 @@ __device__ __forceinline__ int ilog2_ceil(int64_t x) {
     return 64 - __clzll(static_cast<unsigned long long>(x));
 }
 
-// the sum of weight[w] (1 when weight == NULL) over w in N(u) & N(v), computed by the whole warp and returned to
-// every lane: the cheaper of the two intersections above, lane terms in list order, then the fixed butterfly.  The
-// argument order matters only for equal lengths (u's list is then the "shorter" one); callers pass (query, other).
-__device__ __forceinline__ double warp_common_neighbours(const int64_t* __restrict__ rowptr,
-                                                         const int32_t* __restrict__ col,
-                                                         const double* __restrict__ weight, int64_t u, int64_t v,
-                                                         int lane) {
+// The intersection skeleton shared by the sum and the list: N(u) & N(v) walked by the whole warp with the cheaper of
+// the two modes above.  The argument order matters only for equal lengths (u's list is then the "shorter" one);
+// callers pass (query, other).  The visitor sees the common neighbours:
+//   * search: vis.search(hit, w) for each entry w of the shorter list a lane takes, in order.  With
+//     Visitor::kWarpRounds every lane runs every 32-entry round (hit false past the end), so the visitor may ballot;
+//   * merge : vis.merge(walk) once; walk(f) calls f(w) for the lane's common neighbours, in list order, and may be
+//     called more than once.
+template <class Visitor>
+__device__ __forceinline__ void warp_intersect(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                                               int64_t u, int64_t v, int lane, Visitor& vis) {
     int64_t a0 = __ldg(rowptr + u), a1 = __ldg(rowptr + u + 1);
     int64_t b0 = __ldg(rowptr + v), b1 = __ldg(rowptr + v + 1);
     if (a1 - a0 > b1 - b0) {                    // a: the shorter list
@@ -42,37 +45,44 @@ __device__ __forceinline__ double warp_common_neighbours(const int64_t* __restri
     const int64_t la = a1 - a0, lb = b1 - b0;
     const int32_t* A = col + a0;
     const int32_t* B = col + b0;
-    double acc = 0.0;
-    if (la > 0) {
-        const int64_t steps_search = ((la + 31) >> 5) * ilog2_ceil(lb);
-        const int64_t steps_merge = ((la + lb + 31) >> 5) + ilog2_ceil(la);
-        if (steps_search <= steps_merge) {
-            int64_t lo = 0;
-            for (int64_t i = lane; i < la; i += 32) {
-                const int32_t w = __ldg(A + i);
+    if (la == 0) return;
+    const int64_t steps_search = ((la + 31) >> 5) * ilog2_ceil(lb);
+    const int64_t steps_merge = ((la + lb + 31) >> 5) + ilog2_ceil(la);
+    if (steps_search <= steps_merge) {
+        int64_t lo = 0;
+        const int64_t end = Visitor::kWarpRounds ? ((la + 31) & ~int64_t(31)) : la;
+        for (int64_t i = lane; i < end; i += 32) {
+            int32_t w = 0;
+            bool hit = false;
+            if (i < la) {
+                w = __ldg(A + i);
                 int64_t hi = lb;
                 while (lo < hi) {                   // lower bound of w in B[lo, lb)
                     const int64_t m = (lo + hi) >> 1;
                     if (__ldg(B + m) < w) lo = m + 1; else hi = m;
                 }
-                if (lo < lb && __ldg(B + lo) == w) acc += weight ? __ldg(weight + w) : 1.0;
+                hit = lo < lb && __ldg(B + lo) == w;
             }
-        } else {
-            const int64_t L = la + lb;
-            const int64_t d0 = (L * lane) >> 5, d1 = (L * (lane + 1)) >> 5;
-            // i = entries of A among the first d0 of the merge (A first on ties): the largest i with
-            // A[i - 1] <= B[d0 - i]
-            int64_t lo = d0 > lb ? d0 - lb : 0, hi = d0 < la ? d0 : la;
-            while (lo < hi) {
-                const int64_t m = (lo + hi) >> 1;
-                if (__ldg(A + m) <= __ldg(B + d0 - m - 1)) lo = m + 1; else hi = m;
-            }
-            int64_t i = lo, j = d0 - lo;
+            vis.search(hit, w);
+        }
+    } else {
+        const int64_t L = la + lb;
+        const int64_t d0 = (L * lane) >> 5, d1 = (L * (lane + 1)) >> 5;
+        // i = entries of A among the first d0 of the merge (A first on ties): the largest i with
+        // A[i - 1] <= B[d0 - i]
+        int64_t lo = d0 > lb ? d0 - lb : 0, hi = d0 < la ? d0 : la;
+        while (lo < hi) {
+            const int64_t m = (lo + hi) >> 1;
+            if (__ldg(A + m) <= __ldg(B + d0 - m - 1)) lo = m + 1; else hi = m;
+        }
+        const int64_t i_start = lo;
+        vis.merge([&](auto&& f) {
+            int64_t i = i_start, j = d0 - i_start;
             int32_t x = i < la ? __ldg(A + i) : INT32_MAX;
             int32_t y = j < lb ? __ldg(B + j) : INT32_MAX;
             for (int64_t d = d0; d < d1; ++d) {
                 if (i < la && (j >= lb || x <= y)) {
-                    if (x == y) acc += weight ? __ldg(weight + x) : 1.0;
+                    if (x == y) f(x);
                     ++i;
                     x = i < la ? __ldg(A + i) : INT32_MAX;
                 } else {
@@ -80,12 +90,67 @@ __device__ __forceinline__ double warp_common_neighbours(const int64_t* __restri
                     y = j < lb ? __ldg(B + j) : INT32_MAX;
                 }
             }
-        }
+        });
     }
+}
+
+// the sum of weight[w] (1 when weight == NULL): lane terms in list order
+struct SumVisitor {
+    static constexpr bool kWarpRounds = false;
+    const double* __restrict__ weight;
+    double acc;
+    __device__ __forceinline__ void add(int32_t w) { acc += weight ? __ldg(weight + w) : 1.0; }
+    __device__ __forceinline__ void search(bool hit, int32_t w) {
+        if (hit) add(w);
+    }
+    template <class Walk>
+    __device__ __forceinline__ void merge(Walk&& walk) {
+        walk([&](int32_t w) { add(w); });
+    }
+};
+
+// the sum of weight[w] (1 when weight == NULL) over w in N(u) & N(v), computed by the whole warp and returned to
+// every lane: the lane sums of warp_intersect, then the fixed butterfly
+__device__ __forceinline__ double warp_common_neighbours(const int64_t* __restrict__ rowptr,
+                                                         const int32_t* __restrict__ col,
+                                                         const double* __restrict__ weight, int64_t u, int64_t v,
+                                                         int lane) {
+    SumVisitor vis{weight, 0.0};
+    warp_intersect(rowptr, col, u, v, lane, vis);
+    double acc = vis.acc;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
     return acc;
 }
+
+// the list N(u) & N(v) in ascending id order, written to out[0 ..) by the whole warp
+struct ListVisitor {
+    static constexpr bool kWarpRounds = true;
+    int32_t* __restrict__ out;
+    int lane;
+    int64_t base;       // entries written by the rounds before (search) -- warp-uniform
+    __device__ __forceinline__ void search(bool hit, int32_t w) {
+        // the rounds walk the shorter list in order and lane l holds entry l of the round: the hits of the lower
+        // lanes come first
+        const unsigned ballot = __ballot_sync(0xffffffffu, hit);
+        if (hit) out[base + __popc(ballot & ((1u << lane) - 1u))] = w;
+        base += __popc(ballot);
+    }
+    template <class Walk>
+    __device__ __forceinline__ void merge(Walk&& walk) {
+        // lane l's diagonal range follows lane l - 1's: count, exclusive warp scan, write
+        int64_t cnt = 0;
+        walk([&](int32_t) { ++cnt; });
+        int64_t pos = cnt;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int64_t t = __shfl_up_sync(0xffffffffu, pos, o);
+            if (lane >= o) pos += t;
+        }
+        pos = base + pos - cnt;
+        walk([&](int32_t w) { out[pos++] = w; });
+    }
+};
 
 __global__ void __launch_bounds__(kHeurThreads) link_heuristic_kernel(const int64_t* __restrict__ rowptr,
                                                                      const int32_t* __restrict__ col,
@@ -96,8 +161,27 @@ __global__ void __launch_bounds__(kHeurThreads) link_heuristic_kernel(const int6
     const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
     for (int64_t p = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; p < P; p += n_warps) {
         const int64_t u = __ldg(edges + 2 * p), v = __ldg(edges + 2 * p + 1);
-        const double acc = warp_common_neighbours(rowptr, col, weight, u, v, lane);
+        // a negative id (the mean row of BaseModel.encode_for_test) has no neighbours
+        const double acc = u < 0 || v < 0 ? 0.0 : warp_common_neighbours(rowptr, col, weight, u, v, lane);
         if (lane == 0) out[p] = acc;
+    }
+}
+
+// one warp per pair: the common neighbours of edges[p] written to col_out[out_ptr[p] ..), ascending; a pair with a
+// negative id has none
+__global__ void __launch_bounds__(kHeurThreads) common_neighbour_list_kernel(const int64_t* __restrict__ rowptr,
+                                                                            const int32_t* __restrict__ col,
+                                                                            const int64_t* __restrict__ edges,
+                                                                            int64_t P,
+                                                                            const int64_t* __restrict__ out_ptr,
+                                                                            int32_t* __restrict__ col_out) {
+    const int lane = threadIdx.x & 31;
+    const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+    for (int64_t p = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; p < P; p += n_warps) {
+        const int64_t u = __ldg(edges + 2 * p), v = __ldg(edges + 2 * p + 1);
+        if (u < 0 || v < 0) continue;
+        ListVisitor vis{col_out + __ldg(out_ptr + p), lane, 0};
+        warp_intersect(rowptr, col, u, v, lane, vis);
     }
 }
 
@@ -196,8 +280,8 @@ int two_hop_score(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t 
 }  // namespace
 }  // namespace plnlp
 
-// out [P] fp64; rowptr int64 [n + 1] and col int32 [nnz] a cleaned CSR; edges int64 [P, 2] with ids in [0, n);
-// weight fp64 [n] or NULL (CN)
+// out [P] fp64; rowptr int64 [n + 1] and col int32 [nnz] a cleaned CSR; edges int64 [P, 2] with ids in [-1, n) (a
+// pair with a negative id scores 0); weight fp64 [n] or NULL (CN)
 extern "C" int plnlp_link_heuristic_f64(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz,
                                         const double* weight, const int64_t* edges, int64_t P, double* out,
                                         void* stream) {
@@ -208,6 +292,24 @@ extern "C" int plnlp_link_heuristic_f64(const int64_t* rowptr, const int32_t* co
     const int64_t blocks = std::min<int64_t>(plnlp::ceil_div(P, plnlp::kHeurThreads / 32), int64_t(plnlp::kNumSM) * 8);
     plnlp::link_heuristic_kernel<<<static_cast<unsigned>(blocks), plnlp::kHeurThreads, 0,
                                    static_cast<cudaStream_t>(stream)>>>(rowptr, col, weight, edges, P, out);
+    PLNLP_LAUNCH_CHECK();
+    return 0;
+}
+
+// col_out int32 [out_ptr[P]]: the common neighbours of every pair edges[p] (int64 [P, 2], ids in [-1, n)) at
+// col_out[out_ptr[p] .. out_ptr[p + 1]), ascending.  out_ptr int64 [P + 1]: the running sum of the CN counts of
+// plnlp_link_heuristic_f64 (weight NULL), out_ptr[0] = 0.  Same table as above.
+extern "C" int plnlp_common_neighbour_list(const int64_t* rowptr, const int32_t* col, int64_t n, int64_t nnz,
+                                           const int64_t* edges, int64_t P, const int64_t* out_ptr, int32_t* col_out,
+                                           void* stream) {
+    PLNLP_REQUIRE(n >= 0 && nnz >= 0 && P >= 0, PLNLP_E_SIZE);
+    if (P == 0 || nnz == 0) return 0;       // no entries: every list is empty
+    PLNLP_REQUIRE(n > 0, PLNLP_E_SIZE);
+    PLNLP_REQUIRE(rowptr && col && edges && out_ptr && col_out, PLNLP_E_NULL);
+    const int64_t blocks = std::min<int64_t>(plnlp::ceil_div(P, plnlp::kHeurThreads / 32), int64_t(plnlp::kNumSM) * 8);
+    plnlp::common_neighbour_list_kernel<<<static_cast<unsigned>(blocks), plnlp::kHeurThreads, 0,
+                                          static_cast<cudaStream_t>(stream)>>>(rowptr, col, edges, P, out_ptr,
+                                                                               col_out);
     PLNLP_LAUNCH_CHECK();
     return 0;
 }

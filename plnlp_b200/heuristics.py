@@ -41,6 +41,10 @@ sharded mask, select and merge follow.  CN is exact and R = 1 is bit-identical t
 fp32 ulp of one GPU (and, at R >= 3, may differ by an ulp from the partitioned ``score_edges``, whose all-reduce
 sums in another order).  ``RankShard`` is the per-rank step, with no collective.
 
+``common_neighbour_lists`` returns the common neighbours themselves, one ascending list per pair: the count kernel
+of ``score_edges`` (CN) gives the lengths, their running sum the offsets, and a fill kernel with the same
+intersection routine writes the lists.  The NCN predictor (layer.py) sums the embeddings of these nodes.
+
 The path-based scores Katz and Personalized PageRank (``Katz``, ``PPR``, ``PATH_METHODS``) go through the same four
 calls and are run by paths.py, which documents their semantics.
 """
@@ -193,12 +197,18 @@ def shard_table(local, local_t, lo, hi, n, clean=None):
 _CACHE = {}
 
 
+def cached_table(adj):
+    """the ``NeighbourTable`` of ``adj`` if ``neighbour_table`` has built it, else None"""
+    hit = _CACHE.get(id(adj))
+    return hit[1] if hit is not None and hit[0] is adj else None
+
+
 def neighbour_table(adj):
     """the cached ``NeighbourTable`` of an adjacency object (CSRGraph, torch_sparse.SparseTensor) or of this rank's
     block of a ``parallel.ShardedAdj``"""
-    hit = _CACHE.get(id(adj))
-    if hit is not None and hit[0] is adj:
-        return hit[1]
+    hit = cached_table(adj)
+    if hit is not None:
+        return hit
     if isinstance(adj, parallel.ShardedAdj):
         lo, hi = parallel.row_block(adj.n_global, adj.rank, adj.world_size)
         table = shard_table(adj.local, adj.local_t, lo, hi, adj.n_global)
@@ -283,6 +293,43 @@ def score_edges(adj_t, edges, method, batch_size=None):
     for i in starts:
         out[i:i + bs] = shard.partial(e[i:i + bs], method).to(torch.float32)
     return out
+
+
+def _pair_ids(edges, n):
+    """``edges`` checked for ``common_neighbour_lists``: an int64 [P, 2] tensor with ids in [-1, n)"""
+    e = torch.as_tensor(edges)
+    if e.dtype != torch.int64:
+        raise ValueError("edges must be int64")
+    if e.dim() != 2 or e.size(1) != 2:
+        raise ValueError("edges must have shape [P, 2]")
+    if e.numel():
+        lo, hi = torch.stack([e.min(), e.max()]).tolist()          # one host read
+        if lo < -1 or hi >= n:
+            raise ValueError(f"edges: node ids must lie in [-1, {n})")
+    return e
+
+
+def common_neighbour_lists(adj_t, edges):
+    """-> (rowptr int64 [P + 1], col int64 [nnz]) on the adjacency's device: the common neighbours N(u) & N(v) of
+    every pair edges[p] = (u, v) at col[rowptr[p] .. rowptr[p + 1]), in ascending id order (N as in the module
+    docstring; global ids in and out).  ``edges``: int64 [P, 2] with ids in [-1, n); -1 (the mean row of
+    ``BaseModel.encode_for_test``) has no neighbours, and (u, u) lists N(u).  The list lengths are the CN counts of
+    ``score_edges``.  Two host reads: the id range check and the list total.  Raises ValueError for another dtype or shape or an id out of range,
+    NotImplementedError on a row-partitioned graph."""
+    if isinstance(adj_t, parallel.ShardedAdj):
+        raise NotImplementedError("common_neighbour_lists (the NCN predictor) is not implemented on a "
+                                  "row-partitioned graph")
+    e = _pair_ids(edges, _n_nodes(adj_t))
+    table = neighbour_table(adj_t)
+    e = e.to(table.rowptr.device)
+    P = e.size(0)
+    rowptr = torch.zeros(P + 1, dtype=torch.int64, device=e.device)
+    if P:
+        with profiling.span("heuristics: common-neighbour counts"):
+            rowptr[1:] = torch.cumsum(_ops.link_heuristic_raw(table.rowptr, table.col, None, e).to(torch.int64), 0)
+    with profiling.span("heuristics: common-neighbour lists"):
+        col = _ops.common_neighbour_list_raw(table.rowptr, table.col, e, rowptr)
+    return rowptr, col.to(torch.int64)
 
 
 def test(data, split_edge, method, batch_size, evaluator, eval_metric):

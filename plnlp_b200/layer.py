@@ -466,6 +466,57 @@ class MLPPredictor(torch.nn.Module):
         return out
 
 
+class NCNPredictor(torch.nn.Module):
+    """Neural Common Neighbour (Wang, Yang and Zhang, ICLR 2024; an extension, the reference has no such head): the
+    MLP of ``MLPPredictor`` over [h_u * h_v | c_uv], c_uv the sum of h_w over the common neighbours w of u and v
+    (``heuristics.common_neighbour_lists``).  ``lins[0]`` is one Linear(2 H, hidden) whose weight reads as the MLP on
+    the concatenation; the concatenation itself is never built (one GEMM per block into the same output).  Relu +
+    dropout follow every Linear but the last."""
+
+    def __init__(self, in_channels, hidden_channels, out_channels, num_layers, dropout):
+        super().__init__()
+        dims = [2 * in_channels] + [hidden_channels] * (num_layers - 1) + [out_channels]
+        self.lins = torch.nn.ModuleList(_Lin(dims[i], dims[i + 1]) for i in range(num_layers))
+        self.in_channels = in_channels
+        self.dropout = dropout
+
+    def reset_parameters(self):
+        for lin in self.lins:
+            lin.reset_parameters()
+
+    def forward(self, x_i, x_j):
+        raise TypeError("NCNPredictor scores a pair from the graph as well as its two embeddings: call "
+                        "score_edges(h, edges, cn) with cn = heuristics.common_neighbour_lists(adj_t, edges)")
+
+    def score_edges(self, h, edges, cn):
+        """-> [P, out_channels]: the head on h [N, H] for the pairs ``edges`` (rows of h) with ``cn = (rowptr int64
+        [P + 1], col)`` their common-neighbour lists in the row numbering of h"""
+        had = _ops.GatherHadamard.apply(h, edges)
+        c = _ops.common_neighbour_sum(h, cn)
+        H = self.in_channels
+        p = self.dropout if self.training else 0.0
+        first = self.lins[0]
+        W = first.weight
+        if len(self.lins) == 1:
+            if first.out_features == 1:
+                return _ops.MLPOut.apply(had, W[:, :H], first.bias) + _ops.MLPOut.apply(c, W[:, H:], None)
+            return _ops.fused_linear([had, c], [W[:, :H], W[:, H:]], first.bias)
+        x = _ops.fused_linear([had, c], [W[:, :H], W[:, H:]], first.bias, _ops.ACT_RELU, p,
+                              _ops.new_seed() if p > 0 else 0)
+        for lin in self.lins[1:-1]:
+            x = lin(x, act=_ops.ACT_RELU, drop_p=p)
+        last = self.lins[-1]
+        if last.out_features == 1:
+            return _ops.MLPOut.apply(x, last.weight, last.bias)
+        return last(x)
+
+    def flat_params(self):
+        out = []
+        for lin in self.lins:
+            out += [lin.weight, lin.bias]
+        return out
+
+
 class DotPredictor(torch.nn.Module):
     """layer.py:167-176: sum(x_i * x_j, -1) -> [B]."""
 

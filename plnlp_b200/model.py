@@ -20,7 +20,7 @@ import torch
 from . import _ops, profiling
 from .layer import *  # noqa: F401,F403
 from .layer import (GCN, SAGE, WSAGE, BilinearPredictor, DotPredictor, MLPBilPredictor, MLPCatPredictor,
-                    MLPDotPredictor, MLPPredictor, mark_constant)
+                    MLPDotPredictor, MLPPredictor, NCNPredictor, mark_constant)
 from .loss import *  # noqa: F401,F403
 from .utils import *  # noqa: F401,F403
 from .utils import evaluate_hits, evaluate_mrr, get_pos_neg_edges
@@ -34,10 +34,20 @@ PREPARE_AHEAD = os.environ.get("PLNLP_PREPARE_AHEAD", "1") != "0"
 
 
 class PreparedBatch:
-    __slots__ = ("ids", "pos_edge", "neg_edge", "event")
+    __slots__ = ("ids", "pos_edge", "neg_edge", "event", "cn")
 
-    def __init__(self, ids, pos_edge, neg_edge, event):
-        self.ids, self.pos_edge, self.neg_edge, self.event = ids, pos_edge, neg_edge, event
+    def __init__(self, ids, pos_edge, neg_edge, event, cn=None):
+        self.ids, self.pos_edge, self.neg_edge, self.event, self.cn = ids, pos_edge, neg_edge, event, cn
+
+
+def ncn_restrict(edges, cn):
+    """the rows a restricted last conv must compute for the NCN predictor, which reads h at the endpoints AND at
+    their common neighbours: (ids = the sorted union of the ids in ``edges`` [P, 2] and in the lists ``cn =
+    (rowptr, col)``, ``edges`` renumbered into ids, ``(rowptr, col renumbered into ids)``).  ids[edges'] == edges
+    and ids[col'] == col."""
+    rowptr, col = cn
+    ids = torch.unique(torch.cat([edges.reshape(-1), col]))
+    return ids, torch.searchsorted(ids, edges), (rowptr, torch.searchsorted(ids, col))
 
 
 class BaseModel(object):
@@ -141,6 +151,14 @@ class BaseModel(object):
         n_touch = 2 * (pos_edge.size(0) + neg_edge.size(0)) * (self.world_size if self.partitioned else 1)
         return ROW_SPARSE_GRAD and n_touch < 0.5 * self.num_nodes
 
+    def _ncn(self):
+        """is the predictor NCN?  (raises on a row-partitioned model, where it is not implemented)"""
+        if not isinstance(self.predictor, NCNPredictor):
+            return False
+        if self.partitioned:
+            raise NotImplementedError("the NCN predictor is not implemented on a row-partitioned model")
+        return True
+
     def _side(self):
         if getattr(self, "_side_stream", None) is None:
             self._side_stream = torch.cuda.Stream(device=self.device)
@@ -155,20 +173,35 @@ class BaseModel(object):
         edge tensors were themselves produced on the side stream (``run_batches``), so the side stream must NOT wait
         for the main one -- that would queue this work behind the whole step in flight.  Returns None when the batch
         is not row-sparse or the last conv cannot restrict itself (``train_batch`` then does everything itself)."""
+        ncn = self._ncn()
         if not self._sparse_rows(pos_edge, neg_edge):
             return None
         last = self.encoder.convs[-1]
         parts = self.input_parts(data) if len(self.encoder.convs) == 1 else None
         if not (getattr(last, "can_restrict", None) and last.can_restrict(parts, data.adj_t)):
             return None
-        from . import graph
+        from . import graph, heuristics
         main = torch.cuda.current_stream()
         side = self._side()
+        # NCN: the neighbour table is built once per adjacency, on the main stream, and the side stream reads it below,
+        # so the side stream must wait for that build.  Only a build made here is waited for: a prepared batch never
+        # waits for the step in flight.
+        fresh_table = ncn and heuristics.cached_table(data.adj_t) is None
+        if fresh_table:
+            heuristics.neighbour_table(data.adj_t)
         if wait_main:                                            # the edge tensors were produced on the main stream
             side.wait_stream(main)
+        elif fresh_table:
+            built = torch.cuda.Event()
+            built.record(main)
+            side.wait_event(built)
         with torch.cuda.stream(side):
             mine = torch.cat([pos_edge, neg_edge], 0)
-            if self.partitioned:
+            cn = None
+            if ncn:                                              # the list total is read on the side stream too
+                ids, inv, cn = ncn_restrict(mine, heuristics.common_neighbour_lists(data.adj_t, mine))
+                st = graph.structure_of(data.adj_t)
+            elif self.partitioned:
                 from . import parallel
                 if not parallel.RESTRICT_LAST:
                     return None
@@ -183,8 +216,8 @@ class BaseModel(object):
             x_index[ids] = torch.arange(ids.numel(), dtype=torch.int32, device=ids.device)
             ids._plnlp_prepared = {id(st): (plan, x_index)}      # picked up by _ops.SpMMRows
             n_pos = pos_edge.size(0)
-            prep = PreparedBatch(ids, inv[:n_pos], inv[n_pos:], torch.cuda.Event())
-            for t in [ids, inv, x_index] + graph.plan_tensors(plan):
+            prep = PreparedBatch(ids, inv[:n_pos], inv[n_pos:], torch.cuda.Event(), cn)
+            for t in [ids, inv, x_index] + list(cn or ()) + graph.plan_tensors(plan):
                 t.record_stream(main)                            # allocated on the side stream, consumed on the main one
             prep.event.record(side)
         return prep
@@ -201,19 +234,31 @@ class BaseModel(object):
         # in its backward.
         sparse_rows = self._sparse_rows(pos_edge, neg_edge)
         restricted = False
+        ncn = self._ncn()
+        cn = None               # NCN: the common-neighbour lists of [pos_edge; neg_edge], in the row numbering of h
         if self.partitioned:
             from . import parallel
         if prepared is not None:
             torch.cuda.current_stream().wait_event(prepared.event)
             h, restricted = self.encoder(self.input_parts(data), data.adj_t, out_rows=prepared.ids)
             assert restricted
-            pos_edge, neg_edge = prepared.pos_edge, prepared.neg_edge
+            pos_edge, neg_edge, cn = prepared.pos_edge, prepared.neg_edge, prepared.cn
         elif sparse_rows and not self.partitioned:
-            with profiling.span("torch: unique endpoint ids + renumber"):
-                ids, inv = torch.unique(torch.cat([pos_edge, neg_edge], 0), return_inverse=True)
+            mine = torch.cat([pos_edge, neg_edge], 0)
+            if ncn:
+                # h is then read at the endpoints and at their common neighbours: the last conv computes the union
+                from .heuristics import common_neighbour_lists
+                cn = common_neighbour_lists(data.adj_t, mine)
+                with profiling.span("torch: union of endpoint and common-neighbour ids + renumber"):
+                    ids, inv, cn_local = ncn_restrict(mine, cn)
+            else:
+                with profiling.span("torch: unique endpoint ids + renumber"):
+                    ids, inv = torch.unique(mine, return_inverse=True)
             h, restricted = self.encoder(self.input_parts(data), data.adj_t, out_rows=ids)
             if restricted:
                 pos_edge, neg_edge = inv[:pos_edge.size(0)], inv[pos_edge.size(0):]
+                if ncn:
+                    cn = cn_local
         elif sparse_rows and parallel.RESTRICT_LAST:
             # row-partitioned run: the union of every rank's endpoint rows (the same sorted list everywhere) is
             # what the last conv computes -- as partial products over each rank's column block, summed by one
@@ -245,8 +290,13 @@ class BaseModel(object):
                                         head=head, params=self.predictor.flat_params(), drop_p=p,
                                         seed=_ops.new_seed() if p > 0 else 0)
         else:
-            # the other --predictor choices (layer.py:90-189): positives and negatives scored in one pass
-            score = self.predictor.score_edges(h, torch.cat([pos_edge, neg_edge], 0)).reshape(-1)
+            # the other --predictor choices (layer.py:90-189) and NCN: positives and negatives scored in one pass
+            edges = torch.cat([pos_edge, neg_edge], 0)
+            if ncn and cn is None:                   # full h: the lists on the batch's global ids
+                from .heuristics import common_neighbour_lists
+                cn = common_neighbour_lists(data.adj_t, edges)
+            score = (self.predictor.score_edges(h, edges, cn) if ncn
+                     else self.predictor.score_edges(h, edges)).reshape(-1)
             B = pos_edge.size(0)
             loss = _ops.pair_loss(loss_name, score[:B], score[B:], num_neg, weight_margin)
         loss.backward()
@@ -388,9 +438,18 @@ class BaseModel(object):
 
     # ------------------------------------------------------------------
     @torch.no_grad()
-    def batch_predict(self, h, edges, batch_size):
-        """model.py:175-182; scores stay on the device."""
+    def batch_predict(self, h, edges, batch_size, adj_t=None):
+        """model.py:175-182; scores stay on the device.  ``adj_t``: the adjacency whose common neighbours the NCN
+        predictor reads (required for it, unused by the others)."""
         edges = edges.to(self.device)
+        if isinstance(self.predictor, NCNPredictor):
+            if adj_t is None:
+                raise ValueError("batch_predict with the NCN predictor needs adj_t (the graph of the common "
+                                 "neighbours)")
+            from .heuristics import common_neighbour_lists
+            preds = [self.predictor.score_edges(h, e, common_neighbour_lists(adj_t, e)).reshape(-1)
+                     for e in (edges[i:i + batch_size] for i in range(0, edges.size(0), batch_size))]
+            return torch.cat(preds, dim=0) if preds else torch.empty(0, device=self.device)
         preds = [self.predictor.score_edges(h, edges[i:i + batch_size]).reshape(-1)
                  for i in range(0, edges.size(0), batch_size)]
         return torch.cat(preds, dim=0) if preds else torch.empty(0, device=self.device)
@@ -410,15 +469,17 @@ class BaseModel(object):
     @torch.no_grad()
     def test(self, data, split_edge, batch_size, evaluator, eval_metric):
         """model.py:184-226 -> {'Hits@20'|'Hits@50'|'Hits@100'|'MRR': (valid, test)}"""
+        self._ncn()
         self.encoder.eval()
         self.predictor.eval()
         h = self.encode_for_test(data)
         pos_valid_edge, neg_valid_edge = get_pos_neg_edges('valid', split_edge, device=self.device)
         pos_test_edge, neg_test_edge = get_pos_neg_edges('test', split_edge, device=self.device)
-        pos_valid_pred = self.batch_predict(h, pos_valid_edge, batch_size)
-        neg_valid_pred = self.batch_predict(h, neg_valid_edge, batch_size)
-        pos_test_pred = self.batch_predict(h, pos_test_edge, batch_size)
-        neg_test_pred = self.batch_predict(h, neg_test_edge, batch_size)
+        adj = data.adj_t
+        pos_valid_pred = self.batch_predict(h, pos_valid_edge, batch_size, adj_t=adj)
+        neg_valid_pred = self.batch_predict(h, neg_valid_edge, batch_size, adj_t=adj)
+        pos_test_pred = self.batch_predict(h, pos_test_edge, batch_size, adj_t=adj)
+        neg_test_pred = self.batch_predict(h, neg_test_edge, batch_size, adj_t=adj)
         if eval_metric == 'hits':
             return evaluate_hits(evaluator, pos_valid_pred, neg_valid_pred, pos_test_pred, neg_test_pred)
         return evaluate_mrr(evaluator, pos_valid_pred, neg_valid_pred, pos_test_pred, neg_test_pred)
@@ -473,7 +534,7 @@ def create_gnn_layer(input_channels, hidden_channels, num_layers, dropout=0, enc
 
 
 def create_predictor_layer(hidden_channels, num_layers, dropout=0, predictor_name='MLP'):
-    """model.py:263-276 (unknown names -> None, as in the reference)."""
+    """model.py:263-276 (unknown names -> None, as in the reference), plus 'NCN'."""
     name = predictor_name.upper()
     if name == 'DOT':
         return DotPredictor()
@@ -487,6 +548,8 @@ def create_predictor_layer(hidden_channels, num_layers, dropout=0, predictor_nam
         return MLPBilPredictor(hidden_channels, 1, num_layers, dropout)
     if name == 'MLPCAT':
         return MLPCatPredictor(hidden_channels, hidden_channels, 1, num_layers, dropout)
+    if name == 'NCN':             # extension: Neural Common Neighbour (layer.NCNPredictor)
+        return NCNPredictor(hidden_channels, hidden_channels, 1, num_layers, dropout)
     return None
 
 

@@ -38,7 +38,7 @@ from __future__ import annotations
 import torch
 
 from . import _ops, graph, profiling
-from .layer import BilinearPredictor, DotPredictor, MLPBilPredictor, MLPDotPredictor, MLPPredictor
+from .layer import BilinearPredictor, DotPredictor, MLPBilPredictor, MLPDotPredictor, MLPPredictor, NCNPredictor
 
 CHUNK_BYTES = 1 << 30          # default budget of one chunk's score matrix (plus its pair list on the fused MLP path)
 PAIR_PIECE = 1 << 16           # pairs per predictor.score_edges call on the generic path (padded: fixed GEMM shapes)
@@ -87,6 +87,9 @@ class _Scorer:
         self.n_partials = 0
         self.table = h                      # the per-node rows a query reads: what other shards fetch from this one
         dst = None
+        if isinstance(pred, NCNPredictor):
+            raise NotImplementedError("recommend / rank_against_all are not implemented for the NCN predictor (its "
+                                      "score of a pair needs the pair's common neighbours)")
         if isinstance(pred, DotPredictor):
             self.path, dst = "gemm", h[:nb]
         elif isinstance(pred, BilinearPredictor):
