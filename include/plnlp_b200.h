@@ -138,6 +138,7 @@ int plnlp_spmm_csr_bf16(const int32_t* item_ptr, const int32_t* item_row, const 
  *   transb = 0: B[k*ldb + n]     transb = 1: B[n*ldb + k]   (torch Linear weight layout)
  * split_k > 1 needs workspace of split_k*M*N floats; partials are reduced in split order
  * (deterministic).  aux (ldaux) is the forward activation for PLNLP_ACT_RELU_GRAD.
+ * K = 0 gives act(beta * C + bias) and reads neither A nor B (either may be NULL).
  * plnlp_gemm_f32 is the exact-fp32 CUDA-core path (FFMA, fp32 accumulate).
  */
 int plnlp_gemm_f32(int transa, int transb, int64_t M, int64_t N, int64_t K,

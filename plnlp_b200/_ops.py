@@ -158,7 +158,14 @@ def gemm_raw(A, B, transa=False, transb=False, C=None, beta=0.0, bias=None, act=
              drop_p=0.0, seed=0, split_k=None, backend=None, fixed_backend=False):
     """C = act(op(A) @ op(B) + beta*C + bias); A, B row-major with leading dimensions.  ``fixed_backend``: run
     ``backend`` itself, whatever the shape (no switch to the CUDA-core kernel for a small product, no TMA-fed
-    kernel): for a caller whose results must not depend on the row count of A."""
+    kernel): for a caller whose results must not depend on the row count of A.
+
+    A plain-TF32 request ("tf32", "tf32c2") on the CTA kernels runs one pass only when both operands take 16-byte
+    loads (16-byte aligned base, leading dimension and contiguous extent multiples of 4 floats); otherwise they run
+    their scalar-load instantiation, which exists only as 3xTF32.  That result is the "tf32x3" / "tf32x3c2" one bit
+    for bit under the same split_k -- but a plain request keeps its split, it is not raised to TF32X3_KCAP k-terms per
+    accumulator, so with a longer K per split the three passes share one round-toward-zero accumulator.  The TMA-fed
+    tall-skinny kernel (below; it needs only A aligned) splits B itself and runs one pass whatever B's layout."""
     lib = _lib.load()
     A, B = _rowmajor(A), _rowmajor(B)
     M, K = (A.size(1), A.size(0)) if transa else (A.size(0), A.size(1))
@@ -199,7 +206,8 @@ def gemm_raw(A, B, transa=False, transb=False, C=None, beta=0.0, bias=None, act=
                                           float(beta), ptr(bias), int(act), ptr(aux), _ld(aux) if aux is not None else 0,
                                           float(drop_p), int(seed), ptr(wsb), nbytes, stream()), "plnlp_gemm_tf32_tma")
         return C
-    if (backend in ("tf32x3c2", "tf32c2", "tf32x3", "tf32") and GEMM_TMA_TN != "0" and transa and not transb
+    if (backend in ("tf32x3c2", "tf32c2", "tf32x3", "tf32") and GEMM_TMA_TN != "0" and not fixed_backend
+            and transa and not transb
             and M <= 256 and 8 <= N <= 256 and beta == 0.0 and bias is None and act == ACT_NONE
             and _ld(A) % 4 == 0 and _ld(B) % 4 == 0 and A.data_ptr() % 16 == 0 and B.data_ptr() % 16 == 0
             and (GEMM_TMA_TN == "1" or K >= 4 * 148 * TF32X3_KCAP)):
@@ -325,7 +333,9 @@ def row_scatter_raw(g, idx, n_rows):
 
 def fused_edge_mlp_ok(h, params):
     """the fused forward covers the reference recipes' head: MLPPredictor with ONE hidden layer
-    (mlp_num_layers = 2) on a tensor-core backend, hidden width <= 1024"""
+    (mlp_num_layers = 2) on a tensor-core backend, embedding width H <= 1024 (the kernel keeps K = H in one
+    accumulator and rejects more), any hidden width.  H < 32 is left to the unfused path on purpose: the kernel
+    takes it, but gemm_raw runs a layer-1 GEMM with K < 32 on the CUDA cores."""
     if not FUSED_EDGE_MLP or GEMM_BACKEND not in ("tf32x3c2", "tf32c2") or len(params) != 4:
         return False
     W1, w2 = params[0], params[2]
@@ -334,7 +344,10 @@ def fused_edge_mlp_ok(h, params):
 
 
 def edge_mlp_fwd_raw(h, edges, W1, b1, w2, b2, drop_p=0.0, seed=0, need_a1=True):
-    """fused gather + Hadamard + Linear/relu/dropout + Linear(->1): -> (score [P], a1 [P, N1] or None)"""
+    """fused gather + Hadamard + Linear/relu/dropout + Linear(->1): -> (score [P], a1 [P, N1] or None).  With
+    GEMM_BACKEND = "tf32c2" layer 1 runs one TF32 pass only when h and W1 take 16-byte loads (H, both leading
+    dimensions multiples of 4 floats, 16-byte aligned bases); otherwise the scalar gather, which exists only as
+    3xTF32, runs and the result is the "tf32x3c2" one bit for bit."""
     lib = _lib.load()
     h, edges, W1 = _rowmajor(h), _edges_i64(edges), _rowmajor(W1)
     w2 = _f32c(w2).reshape(-1).contiguous()

@@ -239,7 +239,7 @@ extern "C" int plnlp_gemm_tf32(int passes, int transa, int transb, int64_t M, in
     PLNLP_REQUIRE(passes == 1 || passes == 3, PLNLP_E_UNSUPPORTED);
     PLNLP_REQUIRE(M >= 0 && N >= 0 && K >= 0, PLNLP_E_SIZE);
     if (M == 0 || N == 0) return 0;
-    PLNLP_REQUIRE(A && B && C, PLNLP_E_NULL);
+    PLNLP_REQUIRE(C && (K == 0 || (A && B)), PLNLP_E_NULL);     // K = 0 reads neither operand (empty tensors: NULL)
     PLNLP_REQUIRE(lda >= (transa ? M : K) && ldb >= (transb ? K : N) && ldc >= N, PLNLP_E_SIZE);
     PLNLP_REQUIRE(act >= 0 && act <= 2 && drop_p >= 0.0f && drop_p < 1.0f, PLNLP_E_SIZE);
     if (act == PLNLP_ACT_RELU_GRAD) PLNLP_REQUIRE(aux && ldaux >= N, PLNLP_E_NULL);
